@@ -402,6 +402,18 @@ def run_b200(args, rank: int, local_rank: int, world: int):
         wthread.start()
 
     readable = {"rev": 0}
+    # --dump-outputs: countdown[half] counts the timed steps of that half still to come.  The answer of the last one is kept
+    # open (a result stays valid until kb_result_free) to be written after the timed region; every other answer is freed
+    # as usual, so no step runs with more result buffers alive than without the dump.
+    countdown, kept = {"scan": 0, "fan": 0}, {}
+
+    def release(half, res):
+        if countdown[half]:
+            countdown[half] -= 1
+            if countdown[half] == 0:
+                kept[half] = res
+                return
+        res.close()
 
     def fan_device():
         t0 = time.perf_counter()
@@ -409,7 +421,7 @@ def run_b200(args, rank: int, local_rank: int, world: int):
         pyt["cursor"] += time.perf_counter() - t0
         m = weng.watch_match_dev(evh, KB_OUT_DEVICE)
         d = m.n_deliveries
-        m.close()
+        release("fan", m)
         pyt["fan_call"] = pyt.get("fan_call", 0.0) + time.perf_counter() - t0
         return d
 
@@ -441,7 +453,7 @@ def run_b200(args, rank: int, local_rank: int, world: int):
         t2 = time.perf_counter()
         ex = int(r.req_examined.sum())
         nk = r.n_kvs
-        r.close()
+        release("scan", r)
         t3 = time.perf_counter()
         pyt["range_call"] += t2 - t1
         pyt["range_result"] += t3 - t2
@@ -486,7 +498,7 @@ def run_b200(args, rank: int, local_rank: int, world: int):
                 o = (ex, nbytes, checksum)
             else:
                 o = (ex, r.n_kvs)
-            r.close()
+            release("scan", r)
             pyt["range_collect"] += t3 - t2
             pyt["range_result"] += time.perf_counter() - t3
             return o
@@ -562,7 +574,15 @@ def run_b200(args, rank: int, local_rank: int, world: int):
     l0 = sum(e.launch_count() for e in engines)
     for k in list(pyt):
         pyt[k] = 0
+    if args.dump_outputs:
+        countdown.update(scan=args.steps, fan=args.steps)
     dev_ms, wall_s, (examined, n_kvs, deliveries) = timed(False, args.steps)
+    if args.dump_outputs:
+        last = (kept.pop("scan"), kept.pop("fan"))
+        if rank == 0:
+            dump_outputs(args.dump_outputs, eng, *last)
+        for res in last:
+            res.close()
     host_call_us = {k: 1e6 * v / max(pyt["n"], 1) for k, v in pyt.items() if k != "n"}
     launches = sum(e.launch_count() for e in engines) - l0
     prof_major = {}
@@ -843,6 +863,61 @@ def parity_check(eng, weng, wl, evh, reqs, rank: int, world: int, dist):
     return out
 
 
+DUMP_MAX_KVS = 1 << 20  # per-kv arrays: 24 B a kv in the dump
+DUMP_MAX_DELIVERIES = 1 << 21  # delivery list: 4 B a delivery
+DUMP_BYTES_KVS = 2048  # kvs whose key and value bytes are written: ~19 MB at the bench's 2 KB values
+DUMP_LIMIT = 64 << 20
+
+
+def _dump_positions(n: int, cap: int) -> np.ndarray:
+    """all of 0..n-1, or a fixed seeded sorted sample of `cap` of them"""
+    if n <= cap:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(0).choice(n, cap, replace=False))
+
+
+def dump_outputs(out_dir: str, eng, r, m):
+    """Write one step's answers as DIR/<name>.npy (float64 for indices and revisions, float32 for lengths, bytes and
+    delivered event indices) so that two builds can be compared output for output on the same seeded inputs.
+      range_req_first / _count / _examined : per request of the batch
+      range_rec_idx / _rev / _key_len / _val_len : per emitted kv (at the positions range_kv_pos when there are more
+                                                   than DUMP_MAX_KVS)
+      range_bytes_kv, range_key_bytes, range_value_bytes : the key and value bytes of a seeded sample of the emitted kvs,
+                                                   concatenated in sample order (their lengths are in range_*_len)
+      fan_start, fan_event_idx : per-watcher offsets into the delivery list, the delivered event indices (at the positions
+                                 fan_delivery_pos when there are more than DUMP_MAX_DELIVERIES)"""
+    out = {"range_req_first": r.req_first, "range_req_count": r.req_count, "range_req_examined": r.req_examined}
+    r.wait()
+    pos = _dump_positions(r.n_kvs, DUMP_MAX_KVS)
+    if len(pos) < r.n_kvs:
+        out["range_kv_pos"] = pos
+    cols = {name: r.device_array(name, dt)[pos] for name, dt in (
+        ("rec_idx", np.uint32), ("rev", np.uint64), ("key_off", np.uint64), ("key_len", np.uint32),
+        ("val_off", np.uint64), ("val_len", np.uint32))}
+    out["range_rec_idx"], out["range_rev"] = cols["rec_idx"], cols["rev"]
+    out["range_key_len"], out["range_val_len"] = cols["key_len"].astype(np.float32), cols["val_len"].astype(np.float32)
+    pick = _dump_positions(len(pos), DUMP_BYTES_KVS)
+    out["range_bytes_kv"] = pos[pick]
+    for what in ("key", "val"):
+        chunks = [eng.read_device(r.bytes_ptr + int(o), int(n), sync=False)
+                  for o, n in zip(cols[what + "_off"][pick], cols[what + "_len"][pick])]
+        name = "range_key_bytes" if what == "key" else "range_value_bytes"
+        out[name] = np.frombuffer(b"".join(chunks), dtype=np.uint8).astype(np.float32)
+    out["fan_start"] = m.start
+    idx = m.device_event_idx()
+    dpos = _dump_positions(len(idx), DUMP_MAX_DELIVERIES)
+    if len(dpos) < len(idx):
+        out["fan_delivery_pos"] = dpos
+    assert len(idx) == 0 or int(idx.max()) < 1 << 24, "event indices must be exact in float32"
+    out["fan_event_idx"] = idx[dpos].astype(np.float32)
+    out = {k: v if v.dtype == np.float32 else v.astype(np.float64) for k, v in out.items()}
+    total = sum(v.nbytes for v in out.values())
+    assert total <= DUMP_LIMIT, f"dump of {total} bytes exceeds {DUMP_LIMIT}"
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in out.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
+
+
 def latency_probe(eng, wl):
     """SURVEY 8d config 2 latency run: ONE List(limit 10 000) over the whole prefix (backend.List asks the scanner for
     10 001, pkg/backend/range.go:153-171; worker.run stops pulling once the receiver is full).  Reported in microseconds:
@@ -1098,7 +1173,12 @@ def main():
                     help="range batches in flight (kb_range_submit / kb_range_collect); 1 = one kb_range_batch per step, "
                          "joined with the fan-out burst at every step (the round-1 loop)")
     ap.add_argument("--small-compaction", action="store_true", help="extra: config 4 at 1/10 size instead of 100M records")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the range batch and watch match answers of the last timed step (rank "
+                         "0's shard) as DIR/<name>.npy, at most 64 MB; the inputs are seeded, so two builds can be compared")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the answers of the B200 path; the reference arm returns counts only")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
