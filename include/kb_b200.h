@@ -285,7 +285,7 @@ typedef struct kb_prof_entry {
     double   total_ms;
     uint64_t alg_bytes;   /* algorithmic bytes the launches were asked to move (DESIGN.md section 4) */
 } kb_prof_entry;
-int kb_prof_enable(kb_ctx *ctx, int on); /* 0 off, 1 every kernel, 2 only k_decode_lcp and k_gather */
+int kb_prof_enable(kb_ctx *ctx, int on); /* 0 off, 1 every kernel, 2 only k_gather */
 int kb_prof_reset(kb_ctx *ctx);
 int kb_prof_read(kb_ctx *ctx, kb_prof_entry *entries, int cap, int *n);
 uint64_t kb_launch_count(kb_ctx *ctx); /* kernels launched by this ctx since open */

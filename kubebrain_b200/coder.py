@@ -1,7 +1,7 @@
 """Host-side mirror of the reference's internal key codec (pkg/backend/coder/normal.go:25-70, rev.go:22-47).
 
 Only used to build range bounds and to read results; the per-record decode of a scan runs on the GPU
-(k_decode_lcp in csrc/kb_scan.cu).
+(the decoded columns of the record directory, csrc/kb_decode.cuh).
 """
 from __future__ import annotations
 

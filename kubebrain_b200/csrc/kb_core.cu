@@ -6,6 +6,7 @@
 #include <algorithm>
 
 #include "kb_internal.cuh"
+#include "kb_decode.cuh"
 
 // ------------------------------------------------------------------------------------------------
 // errors / buffers
@@ -258,11 +259,9 @@ extern "C" int kb_open(int device_ordinal, const kb_config *cfg, kb_ctx **out)
         cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi) != cudaSuccess)
         prio_lo = prio_hi = 0;
     // three levels when the device has them (numerically lower = more urgent): bound search > lane streams (short kernels of a
-    // batch) > bulk kernels (decode by launch attribute, gather / wire copy by their stream)
+    // batch) > bulk copies (gather / wire copy, by their stream)
     static const bool split = !(getenv("KB_PRIO_SPLIT") && atoi(getenv("KB_PRIO_SPLIT")) == 0);
     prio_lane = (split && prio_lo - prio_hi >= 2) ? prio_lo - 1 : prio_lo;
-    ctx->prio_bulk = prio_lo;
-    ctx->prio_split = prio_lane != prio_lo;
     if (
         cudaStreamCreateWithPriority(&ctx->stream, cudaStreamNonBlocking, high ? prio_hi : prio_lane) != cudaSuccess ||
         // the bound search is tiny and the host waits for it: always ahead of everything; the copy stream (gather / wire
@@ -272,7 +271,7 @@ extern "C" int kb_open(int device_ordinal, const kb_config *cfg, kb_ctx **out)
         cudaEventCreateWithFlags(&ctx->ev_jobs, cudaEventDisableTiming) != cudaSuccess ||
         // second lane of range batches (kb_range_submit) and the stream of the device -> host answer copies
         cudaStreamCreateWithPriority(&ctx->stream_h, cudaStreamNonBlocking, prio_lo) != cudaSuccess ||
-        // work counters of both lanes + the error flag: zeroed once, before any stream can touch them
+        // search counters + the error flag: zeroed once, before any stream can touch them
         cudaMalloc(&ctx->d_ctrs.p, 1024) != cudaSuccess || cudaMemset(ctx->d_ctrs.p, 0, 1024) != cudaSuccess ||
         cudaDeviceSynchronize() != cudaSuccess ||
         cudaEventCreateWithFlags(&ctx->ev_gather[0], cudaEventDisableTiming) != cudaSuccess ||
@@ -283,13 +282,9 @@ extern "C" int kb_open(int device_ordinal, const kb_config *cfg, kb_ctx **out)
     ctx->d_ctrs.cap = 1024;
     // the other lanes of range batches (kb_range_submit): KB_LANES batches in flight at most
     ctx->n_lanes = getenv("KB_LANES") ? std::min(std::max(atoi(getenv("KB_LANES")), 1), KB_MAX_LANES) : 3;
-    ctx->ctr_base = 64;
     ctx->prio_lane = high ? prio_hi : prio_lane;
-    for (int l = 1; l < ctx->n_lanes; l++) {  // their streams are created when a submission first rotates onto them
-        ScanLane &a = ctx->parked[l - 1];
-        a.id = l;
-        a.ctr_base = 64 + 16 * l;
-    }
+    for (int l = 1; l < ctx->n_lanes; l++)  // their streams are created when a submission first rotates onto them
+        ctx->parked[l - 1].id = l;
     *out = ctx;
     return KB_OK;
 }
@@ -318,7 +313,6 @@ void lane_swap(kb_ctx *ctx)
     std::swap(ctx->d_bres, a.d_bres);
     std::swap(ctx->d_reqs, a.d_reqs);
     std::swap(ctx->d_tiles, a.d_tiles);
-    std::swap(ctx->d_meta, a.d_meta);
     std::swap(ctx->d_tgt, a.d_tgt);
     std::swap(ctx->d_tcnt, a.d_tcnt);
     std::swap(ctx->d_tscan, a.d_tscan);
@@ -328,7 +322,6 @@ void lane_swap(kb_ctx *ctx)
     std::swap(ctx->h_stage, a.h_stage);
     std::swap(ctx->h_stage2, a.h_stage2);
     std::swap(ctx->search_pub, a.search_pub);
-    std::swap(ctx->ctr_base, a.ctr_base);
     std::swap(ctx->lane, a.id);
 }
 
@@ -352,7 +345,7 @@ extern "C" void kb_close(kb_ctx *ctx)
     if (ctx->stream_h) cudaStreamSynchronize(ctx->stream_h);
     watch_tables_free(ctx);
     for (auto &a : ctx->parked) {  // (d_tiles aliases d_reqs)
-        DBuf *lane[] = {&a.d_bounds, &a.d_bres, &a.d_reqs, &a.d_meta, &a.d_tgt, &a.d_tcnt, &a.d_tscan, &a.d_reqout, &a.d_sel, &a.d_slot};
+        DBuf *lane[] = {&a.d_bounds, &a.d_bres, &a.d_reqs, &a.d_tgt, &a.d_tcnt, &a.d_tscan, &a.d_reqout, &a.d_sel, &a.d_slot};
         for (DBuf *b : lane) dfree(*b);
         if (a.h_stage.p) cudaFreeHost(a.h_stage.p);
         if (a.h_stage2.p) cudaFreeHost(a.h_stage2.p);
@@ -363,10 +356,11 @@ extern "C" void kb_close(kb_ctx *ctx)
     }
     if (ctx->stream_h) cudaStreamDestroy(ctx->stream_h);
     DBuf *all[] = {&ctx->d_kslab, &ctx->d_koff16, &ctx->d_klen, &ctx->d_vslab, &ctx->d_voff16, &ctx->d_vlen, &ctx->d_dir,
-                   &ctx->d_bounds, &ctx->d_bres, &ctx->d_reqs,
-                   &ctx->d_meta, &ctx->d_tgt, &ctx->d_agg, &ctx->d_tcnt, &ctx->d_tscan, &ctx->d_reqout,
+                   &ctx->d_crev, &ctx->d_cword, &ctx->d_bounds, &ctx->d_bres, &ctx->d_reqs,
+                   &ctx->d_tgt, &ctx->d_agg, &ctx->d_tcnt, &ctx->d_tscan, &ctx->d_reqout,
                    &ctx->d_sel, &ctx->d_slot, &ctx->d_jobs, &ctx->d_gjobs, &ctx->d_jobs2, &ctx->d_gjobs2, &ctx->d_flags, &ctx->d_cursor,
-                   &ctx->d_ctrs, &ctx->s_koff16, &ctx->s_klen, &ctx->s_voff16, &ctx->s_vlen, &ctx->s_dir};
+                   &ctx->d_ctrs, &ctx->s_koff16, &ctx->s_klen, &ctx->s_voff16, &ctx->s_vlen, &ctx->s_dir,
+                   &ctx->s_crev, &ctx->s_cword};
     for (DBuf *b : all) dfree(*b);
     for (auto &b : ctx->free_dev) cudaFree(b.p);
     for (auto &b : ctx->free_host) cudaFreeHost(b.p);
@@ -441,24 +435,19 @@ __global__ void k_repack(const uint8_t *__restrict__ src, const uint64_t *__rest
     }
 }
 
-// strict ascending order of adjacent keys (storage.Iter contract); thread per record
-__global__ void k_check_sorted(StoreDev st, uint32_t *bad)
+// thread per record: the decoded columns (kb_decode.cuh) and the strict ascending order of adjacent keys (storage.Iter
+// contract) in one pass over the keys; bad = the first record that is not greater than its predecessor
+__global__ void __launch_bounds__(256) k_col_build(StoreDev st, uint64_t *__restrict__ crev, uint32_t *__restrict__ cword,
+                                                   uint32_t *__restrict__ bad)
 {
-    uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i == 0 || i >= st.n) return;
-    const uint4 *a = st.kslab + st.koff16[i - 1];
-    const uint4 *b = st.kslab + st.koff16[i];
-    uint32_t la = st.klen[i - 1], lb = st.klen[i];
-    uint32_t m = la < lb ? la : lb;
-    bool less = la < lb;  // all common bytes equal -> shorter first; equal length -> duplicate -> not less
-    for (uint32_t c = 0; c * 16 < m; c++) {
-        uint4 x = a[c], y = b[c];
-        int p = first_diff16(x, y);
-        if (p < 16 && c * 16 + p < m) {
-            less = byte_of(x, p) < byte_of(y, p);
-            break;
-        }
-    }
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= st.n) return;
+    uint64_t r;
+    uint32_t w;
+    bool less;
+    col_entry(st, i, &r, &w, &less);
+    crev[i] = r;
+    cword[i] = w;
     if (!less) atomicMin(bad, i);
 }
 
@@ -468,6 +457,31 @@ __global__ void __launch_bounds__(256) k_pack_dir(StoreDev st, uint4 *__restrict
     if (r >= st.n) return;
     const uint64_t vo = st.voff16[r];
     dir[r] = make_uint4(st.koff16[r], (uint32_t)st.klen[r] | ((uint32_t)(vo >> 32) << 16), st.vlen[r], (uint32_t)vo);
+}
+
+// the decoded columns of the loaded directory, and its key order (KB_EUNSORTED); waits for the device
+static int store_build_columns(kb_ctx *ctx, const char *who)
+{
+    const uint64_t n = ctx->st.n;
+    KB_TRY(dbuf_ensure(ctx, ctx->d_crev, (n + 1) * 8));
+    KB_TRY(dbuf_ensure(ctx, ctx->d_cword, (n + 1) * 4));
+    KB_TRY(dbuf_ensure(ctx, ctx->d_flags, 64));
+    ctx->st.crev = (const uint64_t *)ctx->d_crev.p;
+    ctx->st.cword = (const uint32_t *)ctx->d_cword.p;
+    uint32_t bad = 0xFFFFFFFFu;
+    if (n) {
+        KB_CUDA(ctx, cudaMemcpyAsync(ctx->d_flags.p, &bad, 4, cudaMemcpyHostToDevice, ctx->stream));
+        const uint64_t mean_key = ctx->key_bytes / n;
+        KB_LAUNCH(ctx, "k_col_build", n * (2 * mean_key + 2 * 14 + 16 + 12),  // two keys, two entries, a value probe
+                  (k_col_build<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>(ctx->st, (uint64_t *)ctx->d_crev.p,
+                                                                                    (uint32_t *)ctx->d_cword.p,
+                                                                                    (uint32_t *)ctx->d_flags.p)));
+        KB_CUDA(ctx, cudaGetLastError());
+        KB_CUDA(ctx, cudaMemcpyAsync(&bad, ctx->d_flags.p, 4, cudaMemcpyDeviceToHost, ctx->stream));
+    }
+    KB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    if (bad != 0xFFFFFFFFu) return kb_fail(ctx, KB_EUNSORTED, "%srecord %u is not greater than its predecessor", who, bad);
+    return KB_OK;
 }
 
 int store_pack_dir(kb_ctx *ctx)
@@ -498,10 +512,9 @@ extern "C" int kb_load_sorted(kb_ctx *ctx, const uint8_t *keys, const uint64_t *
     std::vector<uint16_t> klen(n ? n : 1);
     std::vector<uint64_t> voff16(n + 1);
     std::vector<uint32_t> vlen(n ? n : 1);
-    uint64_t kacc = 0, vacc = 0, max_kv = 0, max_k = 0;
+    uint64_t kacc = 0, vacc = 0, max_kv = 0;
     for (uint64_t i = 0; i < n; i++) {
         uint64_t kl = key_off[i + 1] - key_off[i], vl = val_off[i + 1] - val_off[i];
-        max_k = std::max<uint64_t>(max_k, (kl + 15) / 16);
         if (kl > 65535) return kb_fail(ctx, KB_ELIMIT, "key %llu longer than 65535 bytes", (unsigned long long)i);
         if (vl > 0xFFFFFFFFull) return kb_fail(ctx, KB_ELIMIT, "value %llu too long", (unsigned long long)i);
         koff16[i] = (uint32_t)kacc;
@@ -518,7 +531,6 @@ extern "C" int kb_load_sorted(kb_ctx *ctx, const uint8_t *keys, const uint64_t *
     ctx->key_bytes = kacc * 16;
     ctx->val_bytes = vacc * 16;
     ctx->max_kv_chunks = (uint32_t)std::min<uint64_t>(max_kv, 0xFFFFFFFFu);
-    ctx->max_key_chunks = (uint32_t)max_k;
 
     KB_TRY(dbuf_ensure(ctx, ctx->d_kslab, kacc * 16 + 64));
     KB_TRY(dbuf_ensure(ctx, ctx->d_vslab, vacc * 16 + 16));
@@ -602,17 +614,8 @@ extern "C" int kb_load_sorted(kb_ctx *ctx, const uint8_t *keys, const uint64_t *
     ctx->ttl_queue.clear();
     ctx->ttl_of.clear();
 
-    // the iterator contract: strictly ascending unique keys
-    if (n > 1) {
-        KB_TRY(dbuf_ensure(ctx, ctx->d_flags, 64));
-        uint32_t init = 0xFFFFFFFFu, bad = 0;
-        KB_CUDA(ctx, cudaMemcpyAsync(ctx->d_flags.p, &init, 4, cudaMemcpyHostToDevice, ctx->stream));
-        k_check_sorted<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>(ctx->st, (uint32_t *)ctx->d_flags.p);
-        KB_CUDA(ctx, cudaMemcpyAsync(&bad, ctx->d_flags.p, 4, cudaMemcpyDeviceToHost, ctx->stream));
-        KB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-        if (bad != 0xFFFFFFFFu)
-            return kb_fail(ctx, KB_EUNSORTED, "record %u is not greater than its predecessor", bad);
-    }
+    // the decoded columns, and the iterator contract: strictly ascending unique keys
+    KB_TRY(store_build_columns(ctx, ""));
     ctx->loaded = true;
     return KB_OK;
 }
@@ -783,10 +786,9 @@ extern "C" int kb_restore(kb_ctx *ctx, const char *path)
     if (hd != h.sum_dir) return kb_fail(ctx, KB_EINVAL, "restore: directory checksum mismatch");
     // the directory must describe exactly the slabs that follow: monotone offsets, every record inside its slab
     if (koff16[0] != 0 || voff16[0] != 0 || koff16[n] != h.key_chunks || voff16[n] != h.val_chunks) ok = false;
-    uint64_t max_kv = 0, max_k = 0;
+    uint64_t max_kv = 0;
     for (uint64_t i = 0; ok && i < n; i++) {
         const uint64_t nk = ((uint32_t)klen[i] + 15) / 16, nv = ((uint64_t)vlen[i] + 15) / 16;
-        max_k = std::max(max_k, nk);
         if (koff16[i + 1] < koff16[i] || koff16[i + 1] - koff16[i] != nk) ok = false;
         if (voff16[i + 1] < voff16[i] || voff16[i + 1] - voff16[i] != nv) ok = false;
         max_kv = std::max(max_kv, nk + nv);
@@ -817,17 +819,8 @@ extern "C" int kb_restore(kb_ctx *ctx, const char *path)
     ctx->st.vlen = (const uint32_t *)ctx->d_vlen.p;
     ctx->st.n = (uint32_t)n;
     KB_TRY(store_pack_dir(ctx));
-    if (n > 1) {  // the iterator contract, as in kb_load_sorted
-        KB_TRY(dbuf_ensure(ctx, ctx->d_flags, 64));
-        uint32_t init = 0xFFFFFFFFu, bad = 0;
-        KB_CUDA(ctx, cudaMemcpyAsync(ctx->d_flags.p, &init, 4, cudaMemcpyHostToDevice, ctx->stream));
-        k_check_sorted<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>(ctx->st, (uint32_t *)ctx->d_flags.p);
-        KB_CUDA(ctx, cudaMemcpyAsync(&bad, ctx->d_flags.p, 4, cudaMemcpyDeviceToHost, ctx->stream));
-        KB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-        if (bad != 0xFFFFFFFFu) return kb_fail(ctx, KB_EUNSORTED, "restore: record %u is not greater than its predecessor", bad);
-    } else {
-        KB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    }
+    ctx->key_bytes = h.key_chunks * 16;
+    KB_TRY(store_build_columns(ctx, "restore: "));  // the decoded columns and the iterator contract, as in kb_load_sorted
     ctx->kused16 = h.key_chunks;
     ctx->vused16 = h.val_chunks;
     ctx->store_gen++;
@@ -837,7 +830,6 @@ extern "C" int kb_restore(kb_ctx *ctx, const char *path)
     ctx->key_bytes = h.key_chunks * 16;
     ctx->val_bytes = h.val_chunks * 16;
     ctx->max_kv_chunks = (uint32_t)std::min<uint64_t>(max_kv, 0xFFFFFFFFu);
-    ctx->max_key_chunks = (uint32_t)max_k;
     ctx->compact_present = h.compact_present != 0;
     ctx->compact_rev = h.compact_rev;
     ctx->loaded = true;

@@ -1,25 +1,17 @@
-// kb_decode.cuh -- k_decode_lcp: the HBM-bound pass of the scan (included by kb_scan.cu).
+// kb_decode.cuh -- the decoded columns of the record directory and the per-request meta word (included by kb_core.cu
+// and kb_scan.cu).
 //
-// Streams the raw internal keys of every examined record once and reduces each record to one 32-bit meta word:
-//   bits 0..15  LCP with the preceding key (common-prefix length, the input of the "same user key" test)
-//   bits 16..23 decode / visibility / tombstone / compaction-class flags (KB_M_*)
-//
-// Replaces coder.Decode (pkg/backend/coder/normal.go:58-70) and the per-record front half of worker.run
-// (pkg/backend/scanner/scanner.go:430-453, 471-491, 566-591): decode, TTL expiry, revision visibility,
-// tombstone test, deleted-flag revision-record test.  Warps are persistent and fully independent (no CTA barrier).
-//
-// Round 2 layout of the per-warp pipeline.  Round 1 prefetched each lane's packed directory entry, the work ticket and
-// the tile descriptor ONE step ahead into registers; ncu showed every step waiting for exactly those loads
-// (long_scoreboard 43 % at their first use, 101 registers, 12 warps / SM).  Now nothing a step needs arrives through
-// a register-held global load issued less than a block (four steps) earlier:
-//   * work is handed out in BLOCKS of four steps; the ticket (one atomic) for block n+3 and the tile descriptor of block
-//     n+2 are requested when block n starts;
-//   * a step's packed directory entries (16 B per record, plus the record in front of it) are bulk-copied (TMA) into a
-//     three-slot shared-memory ring TWO steps ahead; its key bytes into a two-slot ring ONE step ahead, the copy's extent
-//     read from the directory entries that have just landed; the value probes of 9-byte values (tombstone literal /
-//     deleted-flag revision record) are issued from the same entries one step ahead;
-//   * a step covers K consecutive 32-record sub-tiles of one tile (K chosen per launch from the store's longest key so
-//     that a step always moves ~9 KB: K = 1 at Lk = 269, K = 3 at Lk = 77), each lane looping over its K records.
+// Almost everything coder.Decode (pkg/backend/coder/normal.go:58-70) and the per-record front half of worker.run
+// (pkg/backend/scanner/scanner.go:430-453, 471-491, 566-591) compute about a record is a property of the snapshot, not of
+// the request.  It is computed once, when the directory is written, and kept per record in directory order:
+//   crev  u64  the key's revision when it is non-zero; for a revision record (revision 0) with a value of >= 8 bytes the
+//              BE64 revision in the value's first 8 bytes; 0 otherwise
+//   cword u32  bits 0..15  LCP with the preceding record's key (KB_LCP_INF for record 0)
+//              bits 16..21 static flags: KB_M_DEC_OK, KB_M_REV0, KB_C_TOMBV, KB_C_VL9, KB_C_VL8, KB_C_EVENTS
+// kb_load_sorted / kb_restore build both columns (k_col_build, which also checks the key order), k_dir_merge carries them
+// through a write batch and k_col_fix recomputes the O(ops) entries the batch touched, the layout compaction copies them.
+// A scan turns a record's entry into its meta word (col_meta): only the comparisons against the read revision, the
+// compact revision and timeout_rev are left, so the scan reads 12 bytes per record instead of the record's key.
 #pragma once
 
 #include "kb_internal.cuh"
@@ -27,483 +19,123 @@
 namespace {
 
 constexpr uint32_t MAGIC_LE = 0x8b80fb57u;  // bytes 57 fb 80 8b (coder/normal.go:26)
-constexpr int DECODE_MAX_K = 4;             // sub-tiles (of 32 records) per step
-constexpr uint32_t DECODE_HDR_CHUNKS = 2;   // per directory slot: the step descriptor (32 bytes)
-constexpr int DECODE_MAX_KS = 4;            // key slots per warp (ring depth)
-constexpr int DECODE_MAX_BARS = 2 * DECODE_MAX_KS + 1;  // one mbarrier per key slot and per directory slot
 
-__device__ __forceinline__ uint32_t bswap32(uint32_t x) { return __byte_perm(x, 0, 0x0123); }
-
-// ---- bulk (TMA) copy + mbarrier helpers
-__device__ __forceinline__ uint32_t dsmem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void dmbar_init(uint64_t *bar)
+// bytes.Contains(rawKey, "/events/") for the user key = key bytes [4, len - 9): one 16-byte load per chunk, the bytes
+// shifted through a 64-bit window in registers
+__device__ __forceinline__ bool key_has_events(const uint4 *kp, uint32_t len)
 {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(dsmem_u32(bar)));
-}
-// Bounded wait (a bulk copy that faults never completes its barrier): gives up after ~2 s of polling and raises the
-// context's error flag instead of hanging the stream; the results of that launch are then garbage and the host fails
-// the call (kb_range_batch / kb_compact_sweep check the flag).
-__device__ __forceinline__ bool dmbar_wait(uint64_t *bar, uint32_t parity, unsigned int *err_flag)
-{
-    uint32_t done = 0;
-    for (uint32_t spins = 0; spins < (1u << 26); spins++) {
-        asm volatile(
-            "{\n"
-            ".reg .pred p;\n"
-            "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n"
-            "selp.u32 %0, 1, 0, p;\n"
-            "}\n"
-            : "=r"(done)
-            : "r"(dsmem_u32(bar)), "r"(parity)
-            : "memory");
-        if (done) return true;
-    }
-    atomicExch(err_flag, 1u);
-    return false;
-}
-__device__ __forceinline__ void dbulk_g2s(void *dst, const void *src, uint32_t bytes, uint64_t *bar)
-{
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dsmem_u32(dst)),
-                 "l"(src), "r"(bytes), "r"(dsmem_u32(bar))
-                 : "memory");
-}
-// Streaming variant: the bytes are read once per scan, so they are the first to leave L2 (evict_first) -- the 126 MB L2 then
-// keeps what the latency-bound kernels running beside the scan re-read (directory arrays, meta words, the fan-out's
-// tables and scratch) instead of cycling 1.2 GB of keys and values through it every step.
-__device__ __forceinline__ uint64_t l2_evict_first_policy()
-{
-    uint64_t pol;
-    asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol));
-    return pol;
-}
-__device__ __forceinline__ void dbulk_g2s_stream(void *dst, const void *src, uint32_t bytes, uint64_t *bar, uint64_t pol)
-{
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1], %2, [%3], %4;" ::"r"(
-                     dsmem_u32(dst)),
-                 "l"(src), "r"(bytes), "r"(dsmem_u32(bar)), "l"(pol)
-                 : "memory");
-}
-__device__ __forceinline__ void dmbar_expect(uint64_t *bar, uint32_t bytes)
-{
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(dsmem_u32(bar)), "r"(bytes) : "memory");
-}
-
-// one plain atomic by the calling lane.  Written in PTX because nvcc turns `if (lane == 0) atomicAdd(...)` into its
-// warp-aggregated form, whose result broadcast (SHFL) waits for the atomic at once and defeats issuing it early.
-__device__ __forceinline__ uint32_t atom_add_u32_raw(unsigned int *p, uint32_t v)
-{
-    uint32_t r;
-    asm volatile("atom.global.add.u32 %0, [%1], %2;" : "=r"(r) : "l"(p), "r"(v));
-    return r;
-}
-
-__device__ __forceinline__ bool contains_events(const uint8_t *uk, uint32_t n)  // bytes.Contains(rawKey, "/events/")
-{
+    const uint32_t end = len - 9;
     uint64_t w = 0;
-    for (uint32_t i = 0; i < n; i++) {
-        w = (w << 8) | uk[i];
-        if (i >= 7 && w == 0x2f6576656e74732full) return true;
+    for (uint32_t c = 0; c * 16 < end; c++) {
+        const uint4 x = kp[c];
+#pragma unroll
+        for (int b = 0; b < 16; b++) {
+            const uint32_t p = c * 16 + b;
+            if (p >= 4 && p < end) {
+                w = (w << 8) | byte_of(x, b);
+                if (p >= 11 && w == 0x2f6576656e74732full) return true;
+            }
+        }
     }
     return false;
 }
 
-// One record: LCP with the preceding key + the decode / visibility flags.  kp / pp point at the key and at the key in
-// front of it (shared memory when STAGED, the slab otherwise); v = the first 12 bytes of the value when vl is 9 (or, in
-// the TTL sweep, at least 8).
-template <bool STAGED>
-__device__ __forceinline__ uint32_t decode_record(const ScanMode &mode, uint64_t read_rev, const uint4 *kp, const uint4 *pp,
-                                                  uint32_t len, uint32_t plen, bool has_prev, uint32_t vl, uint32_t vx,
-                                                  uint32_t vy, uint32_t vz)
+// Column entry of record i of `st`, against record i - 1 (none for i == 0).  *less: record i - 1 sorts strictly before
+// record i (bytes.Compare order; always true for i == 0).
+__device__ __forceinline__ void col_entry(const StoreDev &st, uint32_t i, uint64_t *crev, uint32_t *cword, bool *less)
 {
-    const uint8_t *kb = (const uint8_t *)kp;
+    const uint4 *kp = st.kslab + st.koff16[i];
+    const uint32_t len = st.klen[i];
     uint32_t lcp = KB_LCP_INF;
-    if (has_prev) {
-        const uint32_t m = min(len, plen);
-        const uint32_t nch = (m + 15) >> 4;
+    bool lt = true;
+    if (i > 0) {
+        const uint4 *pp = st.kslab + st.koff16[i - 1];
+        const uint32_t plen = st.klen[i - 1];
+        const uint32_t m = min(len, plen), nch = (m + 15) >> 4;
         lcp = m;
-        // four chunks per step; one OR-reduced difference word per chunk, one branch per step.  In the staged
-        // path the loads may run up to three chunks past the shorter key: shared memory is always readable and a
-        // difference found at or beyond m is clamped to m below.
-        for (uint32_t c0 = 0; c0 < nch; c0 += 4) {
+        lt = plen < len;  // all common bytes equal: the shorter key first; equal lengths: a duplicate
+        // four chunk pairs per step, loaded together (the loads stay inside both keys: the index is clamped)
+        bool found = false;
+        for (uint32_t c0 = 0; c0 < nch && !found; c0 += 4) {
             uint4 x[4], y[4];
-            uint32_t dw[4];
 #pragma unroll
             for (int j = 0; j < 4; j++) {
-                const uint32_t c = STAGED ? c0 + j : min(c0 + j, nch - 1);
-                x[j] = kp[c];
-                y[j] = pp[c];
+                const uint32_t c = min(c0 + j, nch - 1);
+                x[j] = pp[c];
+                y[j] = kp[c];
             }
 #pragma unroll
-            for (int j = 0; j < 4; j++)
-                dw[j] = (x[j].x ^ y[j].x) | (x[j].y ^ y[j].y) | (x[j].z ^ y[j].z) | (x[j].w ^ y[j].w);
-            if (dw[0] | dw[1] | dw[2] | dw[3]) {
-                const int j = dw[0] ? 0 : dw[1] ? 1 : dw[2] ? 2 : 3;
-                const uint4 xa = j == 0 ? x[0] : j == 1 ? x[1] : j == 2 ? x[2] : x[3];
-                const uint4 ya = j == 0 ? y[0] : j == 1 ? y[1] : j == 2 ? y[2] : y[3];
-                lcp = min(m, (c0 + j) * 16 + (uint32_t)first_diff16(xa, ya));
-                break;
+            for (int j = 0; j < 4; j++) {
+                const int p = first_diff16(x[j], y[j]);
+                if (!found && c0 + j < nch && p < 16 && (c0 + j) * 16 + p < m) {
+                    lcp = (c0 + j) * 16 + p;
+                    lt = byte_of(x[j], p) < byte_of(y[j], p);
+                    found = true;
+                }
             }
         }
     }
+    const uint8_t *kb = (const uint8_t *)kp;
     uint32_t flags = 0;
-    // coder.Decode (normal.go:58-70); keys shorter than 13 bytes are undecodable (Go would panic)
-    bool dec_ok = len >= 13;
-    if (dec_ok) dec_ok = (((const uint32_t *)kp)[0] == MAGIC_LE) && (kb[len - 9] == 0x24);
-    if (dec_ok) {
-        uint64_t rev;
-        if (STAGED) {
-            // the 8 revision bytes sit at an arbitrary offset: two aligned 64-bit loads + funnel shift + byte swap
-            const uint32_t off = len - 8, sh = (off & 7) * 8;
-            const uint64_t *w = (const uint64_t *)(kb + (off & ~7u));
-            const uint64_t lo = w[0], hi = w[1];
-            const uint64_t le = sh ? (lo >> sh) | (hi << (64 - sh)) : lo;
-            rev = ((uint64_t)bswap32((uint32_t)le) << 32) | bswap32((uint32_t)(le >> 32));
-        } else {
-            rev = be64_bytes(kb + len - 8);
-        }
+    uint64_t r = 0;
+    // coder.Decode; keys shorter than 13 bytes are undecodable (Go would panic)
+    if (len >= 13 && ((const uint32_t *)kp)[0] == MAGIC_LE && kb[len - 9] == 0x24) {
+        const uint64_t rev = be64_bytes(kb + len - 8);
+        const uint32_t vl = st.vlen[i];
+        uint4 v = make_uint4(0, 0, 0, 0);
+        if (vl >= 8) v = st.vslab[st.voff16[i]];
         flags |= KB_M_DEC_OK;
-        if (rev == 0) flags |= KB_M_REV0;
-        const uint64_t vrev = ((uint64_t)bswap32(vx) << 32) | bswap32(vy);
-        bool expired = false;
-        if (mode.ttl_scan && contains_events(kb + 4, len - 13)) {  // compactIfExpired scanner.go:566-591
-            if (rev == 0) {
-                if (vl >= 8 && vrev <= mode.timeout_rev) {
-                    expired = true;
-                    flags |= KB_M_TTLREV;
-                }
-            } else if (rev <= mode.timeout_rev) {
+        r = rev;
+        if (rev == 0) {
+            flags |= KB_M_REV0;
+            if (vl >= 8)  // BE64 of the value's first 8 bytes: the revision a deleted-flag revision record holds
+                r = ((uint64_t)__byte_perm(v.x, 0, 0x0123) << 32) | __byte_perm(v.y, 0, 0x0123);
+        }
+        if (vl == 9) flags |= KB_C_VL9;
+        if (vl >= 8) flags |= KB_C_VL8;
+        if (vl == 9 && v.x == 0x626d6f74u && v.y == 0x6e6f7473u && (v.z & 0xffu) == 0x65u)
+            flags |= KB_C_TOMBV;  // "tombstone" util.go:28
+        if (key_has_events(kp, len)) flags |= KB_C_EVENTS;
+    }
+    *crev = r;
+    *cword = lcp | flags;
+    *less = lt;
+}
+
+// The meta word of one record for one request: LCP (KB_LCP_INF for the request's first record, which has no predecessor
+// inside the request) + the decode / visibility / tombstone / compaction-class flags (KB_M_*).
+__device__ __forceinline__ uint32_t col_meta(uint64_t crev, uint32_t cword, const ScanMode &mode, uint64_t read_rev,
+                                             bool first)
+{
+    uint32_t w = first ? KB_LCP_INF : (cword & KB_M_LCP_MASK);
+    if (!(cword & KB_M_DEC_OK)) return w;
+    w |= cword & (KB_M_DEC_OK | KB_M_REV0);
+    const bool rev0 = (cword & KB_M_REV0) != 0;
+    bool expired = false;
+    if (mode.ttl_scan && (cword & KB_C_EVENTS)) {  // compactIfExpired scanner.go:566-591
+        if (rev0) {
+            if ((cword & KB_C_VL8) && crev <= mode.timeout_rev) {
                 expired = true;
-                flags |= KB_M_TTLOBJ;
+                w |= KB_M_TTLREV;
             }
-        }
-        if (!expired && rev <= read_rev) {  // scanner.go:451-453
-            flags |= KB_M_TRIG;
-            if (vl == 9 && vx == 0x626d6f74u && vy == 0x6e6f7473u && (vz & 0xffu) == 0x65u)
-                flags |= KB_M_TOMB;  // "tombstone" util.go:28
-            bool prevok = true;
-            if (mode.compact && rev == 0 && vl == 9) {  // scanner.go:476-491
-                if (vrev > read_rev)
-                    prevok = false;  // `continue` without updating prev (Q5)
-                else
-                    flags |= KB_M_REVDEL;
-            }
-            if (prevok) flags |= KB_M_PREVOK;
+        } else if (crev <= mode.timeout_rev) {
+            expired = true;
+            w |= KB_M_TTLOBJ;
         }
     }
-    return lcp | flags;
-}
-
-// launch geometry (chosen by the host from the longest key of the store, see decode_geometry)
-struct DecGeom {
-    uint32_t K;          // 32-record sub-tiles per step
-    uint32_t SK;         // key chunks per key-ring slot: (32 K + 1) keys of the longest length
-    uint32_t DS;         // chunks per directory slot: 32 K + 1 entries + DECODE_HDR_CHUNKS
-    uint32_t NKS;        // key slots per warp (keys in flight NKS - 1 steps ahead); NKS + 1 directory slots
-    uint32_t warps;      // warps per CTA
-    uint32_t bpt;        // blocks (of four steps) per tile: ceil(ceil(32 / K) / 4)
-    uint32_t n_blocks;   // tiles * bpt
-};
-
-// step descriptor, written by lane 0 into the head of the step's directory slot
-struct StepHdr {
-    uint32_t r0, nrec, flat, halo;   // first record, records, first meta slot, 1: the entry in front of r0 is staged too
-    uint32_t rr_lo, rr_hi;           // read revision of the request
-    uint32_t base16, span;           // key chunk interval (filled when the key copy is issued); span == ~0u: last step
-};
-static_assert(sizeof(StepHdr) == DECODE_HDR_CHUNKS * 16, "StepHdr is the slot header");
-
-struct BlockTile {
-    uint32_t valid, rec0, n, flat0, first /* rec0 is the request's first record */, bj /* block inside the tile */;
-    uint32_t rr_lo, rr_hi;
-};
-
-__device__ __forceinline__ BlockTile make_block(uint32_t b, const DecGeom &g, const uint4 &ta, const uint4 &tb)
-{
-    BlockTile t;
-    t.valid = b < g.n_blocks;
-    t.rec0 = ta.y;
-    t.n = ta.z;
-    t.flat0 = ta.w;
-    t.first = ta.y == tb.x;  // TileDev.rec0 == TileDev.lo
-    t.bj = b % g.bpt;
-    t.rr_lo = tb.z;
-    t.rr_hi = tb.w;
-    return t;
-}
-
-template <int MAXW, int KK>
-// Register budget: the decode CTA shares its SM with the fan-out context's persistent CTA (384 threads x 64) and with the
-// short kernels of other range batches in flight (256 threads x 32); at 96 registers x 12 warps they did not fit together
-// and waited for each other.  The long-key variant (K = 1) is the one that runs beside them.
-__global__ void __maxnreg__((KK == 1 || MAXW > 16) ? 80 : 128)
-k_decode_lcp(StoreDev st, const TileDev *__restrict__ tiles, DecGeom g, ScanMode mode, uint32_t *__restrict__ meta,
-             unsigned int *__restrict__ work_ctr, unsigned int *__restrict__ err_flag)
-{
-    extern __shared__ uint4 smem[];  // per warp: key slots[NKS][SK] | directory slots[NKS + 1][DS]
-    __shared__ uint64_t bars[MAXW * DECODE_MAX_BARS];
-    const uint32_t warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const unsigned FULLM = 0xffffffffu;
-    const uint32_t NKS = g.NKS, NDS = g.NKS + 1;  // a step's keys are in flight NKS - 1 steps, its directory entries NKS
-    const uint64_t l2pol = l2_evict_first_policy();
-    uint4 *kbuf = smem + (size_t)warp * (NKS * g.SK + NDS * g.DS);
-    uint4 *dbuf = kbuf + NKS * g.SK;
-    uint64_t *kbar = bars + warp * DECODE_MAX_BARS, *dbar = kbar + DECODE_MAX_KS;
-    if (lane == 0) {
-        for (int i = 0; i < DECODE_MAX_BARS; i++) dmbar_init(kbar + i);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    if (!expired && (rev0 || crev <= read_rev)) {  // scanner.go:451-453
+        w |= KB_M_TRIG;
+        if (cword & KB_C_TOMBV) w |= KB_M_TOMB;
+        bool prevok = true;
+        if (mode.compact && rev0 && (cword & KB_C_VL9)) {  // scanner.go:476-491
+            if (crev > read_rev)
+                prevok = false;  // `continue` without updating prev (Q5)
+            else
+                w |= KB_M_REVDEL;
+        }
+        if (prevok) w |= KB_M_PREVOK;
     }
-    __syncwarp();
-
-    // ---- block stream of this warp: the first three blocks are static (they fill the pipeline), the rest come from the
-    // global counter (left at zero by k_emit_place, which follows every decode pass), so a CTA that starts late -- its SM
-    // was still busy with another stream's kernel -- simply takes fewer.
-    const uint32_t stride = gridDim.x * g.warps;
-    const uint32_t dyn_base = 3 * stride;
-    auto tile_of = [&](uint32_t b, uint4 &ta, uint4 &tb) {
-        ta = tb = make_uint4(0, 0, 0, 0);
-        if (b < g.n_blocks) {
-            const uint4 *p = (const uint4 *)(tiles + b / g.bpt);
-            ta = __ldg(p);
-            tb = __ldg(p + 1);
-        }
-    };
-    uint32_t b0 = blockIdx.x * g.warps + warp;
-    uint4 la, lb;
-    tile_of(b0, la, lb);
-    BlockTile T = make_block(b0, g, la, lb);           // block the generator is in
-    uint32_t b1 = b0 + stride;
-    tile_of(b1, la, lb);
-    BlockTile Tn = make_block(b1, g, la, lb);          // the block after it
-    uint32_t b2 = b1 + stride;                         // block whose tile descriptor is in flight (la, lb)
-    tile_of(b2, la, lb);
-    uint32_t raw = 0;                                  // lane 0: ticket of the block after b2
-    if (lane == 0) raw = atom_add_u32_raw(work_ctr, 1u);
-    uint32_t gj = 0;                                   // generator: step inside its block (0..3)
-
-    // generator: describe the next step of the stream in directory slot `slot` and start the copy of its entries
-    auto generate = [&](uint32_t slot) {
-        uint4 *ds = dbuf + (size_t)slot * g.DS;
-        StepHdr *h = (StepHdr *)ds;
-        uint32_t nrec = 0, r0 = 0, flat = 0, halo = 0;
-        const bool live = T.valid != 0;
-        if (live) {
-            const uint32_t sub0 = (T.bj * 4 + gj) * KK;
-            if (sub0 * 32 < T.n) {
-                nrec = min((uint32_t)KK * 32, T.n - sub0 * 32);
-                r0 = T.rec0 + sub0 * 32;
-                flat = T.flat0 + sub0 * 32;
-                halo = (T.first && sub0 == 0) ? 0u : 1u;
-            }
-        }
-        if (lane == 0) {
-            h->r0 = r0;
-            h->nrec = nrec;
-            h->flat = flat;
-            h->halo = halo;
-            h->rr_lo = T.rr_lo;
-            h->rr_hi = T.rr_hi;
-            h->base16 = 0;
-            h->span = live ? 0u : ~0u;
-            if (nrec) {
-                // the slot was last read (generic proxy) three steps ago; the __syncwarp that ended that step orders
-                // those reads before this point, the proxy fence orders them before the async-proxy write
-                asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-                const uint32_t bytes = (nrec + halo) * 16;
-                dmbar_expect(dbar + slot, bytes);
-                dbulk_g2s(ds + DECODE_HDR_CHUNKS, st.dir + (r0 - halo), bytes, dbar + slot);
-            }
-        }
-        if (live && ++gj == 4) {  // enter the next block: everything it needs was requested a block ago
-            gj = 0;
-            T = Tn;
-            Tn = make_block(b2, g, la, lb);
-            b2 = dyn_base + __shfl_sync(FULLM, raw, 0);
-            tile_of(b2, la, lb);
-            if (lane == 0) raw = atom_add_u32_raw(work_ctr, 1u);
-        }
-    };
-
-    uint32_t vx[KK], vy[KK], vz[KK];    // value probes of the step being processed
-    uint32_t nx[KK], ny[KK], nz[KK];    // ... of the step whose keys are in flight
-#pragma unroll
-    for (int k = 0; k < KK; k++) vx[k] = vy[k] = vz[k] = nx[k] = ny[k] = nz[k] = 0;
-    uint32_t phase = 0;  // bit i: parity of the next completion of barrier i (key slots 0 .., directory slots DECODE_MAX_KS ..)
-
-    // keys + value probes of the step described in directory slot `slot`, into key slot `ks`
-    auto stage_keys = [&](uint32_t slot, uint32_t ks) {
-        uint4 *ds = dbuf + (size_t)slot * g.DS;
-        StepHdr *h = (StepHdr *)ds;
-        const uint32_t nrec = h->nrec, halo = h->halo;
-        if (nrec == 0) return;
-        dmbar_wait(dbar + slot, (phase >> (DECODE_MAX_KS + slot)) & 1, err_flag);
-        phase ^= 1u << (DECODE_MAX_KS + slot);
-        const uint4 *ent = ds + DECODE_HDR_CHUNKS;
-        const uint32_t cnt = nrec + halo;
-        // Chunk interval covering every key of the step (and the one in front of it).  In a freshly loaded or compacted
-        // store the keys of consecutive records are contiguous and this is exactly first .. last; records appended by
-        // kb_apply_batch since then live at the slab tail, the interval then exceeds the ring slot and the step reads its
-        // keys in place (unstaged path).
-        uint32_t lo16 = 0xFFFFFFFFu, hi16 = 0;
-#pragma unroll
-        for (int k = 0; k <= KK; k++) {
-            const uint32_t r = k * 32 + lane;
-            if (r < cnt) {
-                const uint4 e = ent[r];
-                lo16 = min(lo16, e.x);
-                hi16 = max(hi16, e.x + (((e.y & 0xffffu) + 15) >> 4));
-            }
-        }
-        const uint32_t base16 = __reduce_min_sync(FULLM, lo16);
-        const uint32_t span = __reduce_max_sync(FULLM, hi16) - base16;
-        if (lane == 0) {
-            h->base16 = base16;
-            h->span = span;
-            if (span <= g.SK) {
-                asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-                dmbar_expect(kbar + ks, span * 16);
-                dbulk_g2s_stream(kbuf + (size_t)ks * g.SK, st.kslab + base16, span * 16, kbar + ks, l2pol);
-            }
-        }
-    };
-
-    // value probes of the step described in directory slot `slot` (its entries landed when its keys were staged): issued one
-    // step before the step is decoded.  Only 9-byte values are ever inspected by the range path; the TTL sweep also reads
-    // revision-record values.
-    auto probe_values = [&](uint32_t slot) {
-        const uint4 *ds = dbuf + (size_t)slot * g.DS;
-        const StepHdr *h = (const StepHdr *)ds;
-        const uint32_t nrec = h->nrec, halo = h->halo;
-        const uint4 *ent = ds + DECODE_HDR_CHUNKS;
-#pragma unroll
-        for (int k = 0; k < KK; k++) {
-            nx[k] = ny[k] = nz[k] = 0;
-            const uint32_t r = k * 32 + lane;
-            if (r < nrec) {
-                const uint4 e = ent[halo + r];
-                const uint32_t vl = e.z;
-                if (vl >= 8 && (vl == 9 || mode.ttl_scan)) {
-                    const uint4 v = __ldg(st.vslab + (((uint64_t)(e.y >> 16) << 32) | e.w));
-                    nx[k] = v.x;
-                    ny[k] = v.y;
-                    nz[k] = v.z;
-                }
-            }
-        }
-    };
-
-    // decode the step in directory slot `slot` whose keys were staged into key slot `ks`; false: end of the stream
-    auto process = [&](uint32_t slot, uint32_t ks) -> bool {
-        const uint4 *ds = dbuf + (size_t)slot * g.DS;
-        const StepHdr *h = (const StepHdr *)ds;
-        const uint32_t nrec = h->nrec;
-        if (nrec == 0) return h->span != ~0u;
-        const uint32_t halo = h->halo, base16 = h->base16, span = h->span;
-        const uint64_t read_rev = ((uint64_t)h->rr_hi << 32) | h->rr_lo;
-        const bool staged = span <= g.SK;
-        if (staged) {
-            dmbar_wait(kbar + ks, (phase >> ks) & 1, err_flag);
-            phase ^= 1u << ks;
-        }
-        const uint4 *ent = ds + DECODE_HDR_CHUNKS + halo;  // ent[r] = record r0 + r; ent[-1] = the record in front (halo)
-        const uint4 *buf = kbuf + (size_t)ks * g.SK;
-#pragma unroll
-        for (int k = 0; k < KK; k++) {
-            const uint32_t r = k * 32 + lane;
-            if (r < nrec) {
-                const uint4 e = ent[r];
-                const bool has_prev = halo != 0 || r > 0;
-                uint4 pe = e;
-                if (has_prev) pe = ent[(int)r - 1];
-                const uint32_t kl = e.y & 0xffffu, pkl = pe.y & 0xffffu;
-                uint32_t word;
-                if (staged)
-                    word = decode_record<true>(mode, read_rev, buf + (e.x - base16), buf + (pe.x - base16), kl, pkl, has_prev,
-                                               e.z, vx[k], vy[k], vz[k]);
-                else
-                    word = decode_record<false>(mode, read_rev, st.kslab + e.x, st.kslab + pe.x, kl, pkl, has_prev, e.z,
-                                                vx[k], vy[k], vz[k]);
-                meta[h->flat + r] = word;
-            }
-        }
-        return true;
-    };
-
-    // prologue: steps 0 .. NKS-1 described, keys of steps 0 .. NKS-2 in flight, probes of step 0 issued
-    for (uint32_t i = 0; i < NKS; i++) {
-        generate(i);
-        __syncwarp();
-    }
-    for (uint32_t i = 0; i + 1 < NKS; i++) stage_keys(i, i);
-    probe_values(0);
-#pragma unroll
-    for (int k = 0; k < KK; k++) {
-        vx[k] = nx[k];
-        vy[k] = ny[k];
-        vz[k] = nz[k];
-    }
-    __syncwarp();
-    // steady state, iteration i: describe step i+NKS, stage the keys of step i+NKS-1, probe the values of step i+1, decode
-    // step i.  d0 / k0: directory / key slot of the step being decoded.
-    uint32_t d0 = 0, k0 = 0;
-    for (;;) {
-        const uint32_t dg = d0 + NKS >= NDS ? d0 + NKS - NDS : d0 + NKS;       // (d0 + NKS) mod NDS
-        const uint32_t dk = d0 + NKS - 1 >= NDS ? d0 - 2 : d0 + NKS - 1;        // (d0 + NKS - 1) mod NDS
-        const uint32_t kk = k0 == 0 ? NKS - 1 : k0 - 1;                         // (k0 + NKS - 1) mod NKS
-        const uint32_t d1 = d0 + 1 == NDS ? 0 : d0 + 1;
-        generate(dg);
-        __syncwarp();
-        stage_keys(dk, kk);
-        probe_values(d1);
-        const bool more = process(d0, k0);
-#pragma unroll
-        for (int k = 0; k < KK; k++) {
-            vx[k] = nx[k];
-            vy[k] = ny[k];
-            vz[k] = nz[k];
-        }
-        __syncwarp();
-        if (!more) break;
-        d0 = d1;
-        k0 = k0 + 1 == NKS ? 0 : k0 + 1;
-    }
-}
-
-// geometry for a store whose longest key has `max_key_chunks` 16-byte chunks; K, the ring depth and the warp count can
-// be forced for experiments (KB_DECODE_K, KB_DECODE_NKS, KB_DECODE_WARPS)
-static inline DecGeom decode_geometry(uint32_t max_key_chunks, uint32_t ntiles, uint32_t force_k, uint32_t force_nks,
-                                      uint32_t force_warps, size_t *smem_bytes)
-{
-    const uint32_t c = std::max<uint32_t>(max_key_chunks, 1);
-    const size_t budget = 227 * 1024 - 2048;
-    DecGeom g;
-    uint32_t K = force_k ? force_k : (c >= 9 ? 1u : c >= 5 ? 2u : 4u);
-    K = std::min<uint32_t>(std::max<uint32_t>(K, 1), DECODE_MAX_K);
-    // Ring depth.  Measured (profiles/r02_run2_decode_sweep.txt, 1M records of 269 B): 2 key slots x 11 warps 59 us, 3 x 7
-    // 77 us, 4 x 5 98 us -- the pass is bound by how many warps decode, not by the bytes in flight, so the shallowest ring
-    // (most warps) is the default.
-    uint32_t NKS = force_nks ? std::min<uint32_t>(std::max<uint32_t>(force_nks, 2), DECODE_MAX_KS) : 2;
-    auto per_warp = [&](uint32_t k, uint32_t nks) {
-        return (size_t)(nks * (32 * k + 1) * c + (nks + 1) * (32 * k + 1 + DECODE_HDR_CHUNKS)) * 16;
-    };
-    while (per_warp(K, NKS) * 4 > budget && NKS > 2) NKS--;
-    while (per_warp(K, NKS) * 4 > budget && K > 1) K--;  // very long keys: fewer records per step rather than < 4 warps
-    g.K = K;
-    g.NKS = NKS;
-    g.DS = 32 * K + 1 + DECODE_HDR_CHUNKS;
-    g.SK = (32 * K + 1) * c;
-    // keys longer than ~1.7 KB: the ring would not hold a sub-tile even with four warps; cap the slot, such steps take
-    // the unstaged path (direct loads from the slab)
-    const uint32_t max_sk = (uint32_t)((budget / 4 / 16 - (NKS + 1) * g.DS) / NKS);
-    g.SK = std::min(g.SK, max_sk);
-    const size_t pw = (size_t)(NKS * g.SK + (NKS + 1) * g.DS) * 16;
-    uint32_t warps = (uint32_t)std::min<size_t>(budget / pw, 24);
-    if (force_warps) warps = std::min(warps, force_warps);
-    g.warps = std::max<uint32_t>(warps, 1);
-    const uint32_t spt = (32 + K - 1) / K;
-    g.bpt = (spt + 3) / 4;
-    g.n_blocks = ntiles * g.bpt;
-    *smem_bytes = pw * g.warps;
-    return g;
+    return w;
 }
 
 }  // namespace

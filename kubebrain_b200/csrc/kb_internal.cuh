@@ -25,8 +25,10 @@ struct StoreDev {
     const uint4    *vslab;   // values, 16-byte aligned, zero padded
     const uint64_t *voff16;  // n+1 offsets in 16-byte units
     const uint32_t *vlen;    // n exact value lengths
-    const uint4    *dir;     // n packed directory entries for the decode pass (one 16-byte load per record):
+    const uint4    *dir;     // n packed directory entries (one 16-byte load per record):
                              // {koff16, klen | (voff16 >> 32) << 16, vlen, (uint32_t)voff16}
+    const uint64_t *crev;    // n decoded columns (kb_decode.cuh): revision of the key, or of a revision record's value
+    const uint32_t *cword;   //   LCP with the preceding key | static flags (KB_C_*)
     uint32_t        n;
 };
 
@@ -51,7 +53,7 @@ struct TileDev {
     uint32_t rec0;   // first store record of the tile
     uint32_t n;      // records in the tile (<= TILE)
     uint32_t flat0;  // flat slot of rec0
-    uint32_t lo;     // first record of the request (copy of ReqDev.lo: one load instead of two in the decode pass)
+    uint32_t lo;     // first record of the request (copy of ReqDev.lo)
     uint32_t pad;
     uint64_t read_rev;
 };
@@ -64,7 +66,7 @@ struct ScanMode {
 };
 enum { KB_WIRE_NONE_I = 0, KB_WIRE_KVS_I = 1, KB_WIRE_EVENTS_I = 2 };
 
-// per-record meta word produced by the decode pass
+// per-record meta word of one request (col_meta, kb_decode.cuh)
 #define KB_M_LCP_MASK 0x0000FFFFu
 #define KB_M_DEC_OK   (1u << 16)
 #define KB_M_REV0     (1u << 17)   // revision == 0 (revision record)
@@ -74,6 +76,12 @@ enum { KB_WIRE_NONE_I = 0, KB_WIRE_KVS_I = 1, KB_WIRE_EVENTS_I = 2 };
 #define KB_M_REVDEL   (1u << 21)   // class 3 victim
 #define KB_M_TTLREV   (1u << 22)   // class 4 victim
 #define KB_M_TTLOBJ   (1u << 23)   // class 5 victim
+// static flags of a record's column word (cword bits 16..21; DEC_OK and REV0 keep their meta-word positions)
+#define KB_C_TOMBV    (1u << 18)   // value == "tombstone"
+#define KB_C_VL9      (1u << 19)   // value length == 9
+#define KB_C_VL8      (1u << 20)   // value length >= 8
+#define KB_C_EVENTS   (1u << 21)   // the user key contains "/events/"
+#define KB_C_FLAGS    (KB_M_DEC_OK | KB_M_REV0 | KB_C_TOMBV | KB_C_VL9 | KB_C_VL8 | KB_C_EVENTS)
 #define KB_LCP_INF    0xFFFFu
 #define KB_NONE       0xFFFFFFFFu
 
@@ -125,6 +133,39 @@ __device__ __forceinline__ uint64_t be64_bytes(const uint8_t *p)
 
 __device__ __forceinline__ uint32_t pad16(uint32_t x) { return (x + 15u) & ~15u; }
 
+// ---- mbarrier / bulk-copy helpers of the TMA copies (k_gather, k_wire_copy)
+__device__ __forceinline__ uint32_t dsmem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
+// Bounded wait (a bulk copy that faults never completes its barrier): gives up after ~2 s of polling and raises the
+// context's error flag instead of hanging the stream; the results of that launch are then garbage and the host fails
+// the call (kb_range_batch checks the flag).
+__device__ __forceinline__ bool dmbar_wait(uint64_t *bar, uint32_t parity, unsigned int *err_flag)
+{
+    uint32_t done = 0;
+    for (uint32_t spins = 0; spins < (1u << 26); spins++) {
+        asm volatile(
+            "{\n"
+            ".reg .pred p;\n"
+            "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n"
+            "selp.u32 %0, 1, 0, p;\n"
+            "}\n"
+            : "=r"(done)
+            : "r"(dsmem_u32(bar)), "r"(parity)
+            : "memory");
+        if (done) return true;
+    }
+    atomicExch(err_flag, 1u);
+    return false;
+}
+// Streaming copies: the bytes are read once per answer, so they are the first to leave L2 (evict_first) -- the 126 MB L2
+// then keeps what the latency-bound kernels running beside the copy re-read (directory arrays, decoded columns, the
+// fan-out's tables and scratch) instead of cycling the answer's keys and values through it every step.
+__device__ __forceinline__ uint64_t l2_evict_first_policy()
+{
+    uint64_t pol;
+    asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol));
+    return pol;
+}
+
 // ------------------------------------------------------------------------------------------------
 // host plumbing
 // ------------------------------------------------------------------------------------------------
@@ -173,10 +214,9 @@ struct ScanLane {
     uint8_t *h_rout = nullptr;
     size_t h_rout_cap = 0;
     uint64_t rout_epoch = 0;
-    DBuf d_bounds, d_bres, d_reqs, d_tiles, d_meta, d_tgt, d_tcnt, d_tscan, d_reqout, d_sel, d_slot;
+    DBuf d_bounds, d_bres, d_reqs, d_tiles, d_tgt, d_tcnt, d_tscan, d_reqout, d_sel, d_slot;
     HBuf h_stage, h_stage2;
     SearchPubBuf search_pub;
-    uint32_t ctr_base = 0;   // this lane's work counters inside d_ctrs
     int id = 0;
 };
 constexpr int KB_MAX_LANES = 4;
@@ -187,7 +227,7 @@ struct kb_ctx {
     int device = 0;
     cudaStream_t stream = nullptr;
     cudaStream_t stream2 = nullptr;  // bound search of a range batch: runs beside the tail (gather) of the previous batch
-    // The gather / wire copy of a range batch runs on its own stream, so the next batch's decode .. placement (main
+    // The gather / wire copy of a range batch runs on its own stream, so the next batch's emit .. placement (main
     // stream) overlaps it.  Two sets of job buffers alternate between consecutive batches; ev_gather[set] marks the end
     // of the last gather that read a set, ev_jobs the end of the current batch's job construction.
     cudaStream_t stream_g = nullptr;
@@ -196,11 +236,8 @@ struct kb_ctx {
     ScanLane parked[KB_MAX_LANES - 1];            // the other lanes (kb_range_submit rotates through them)
     int n_lanes = 2, park_next = 0;
     int lane = 0;                                 // which lane the context's own fields are right now
-    uint32_t ctr_base = 0;                        // the current lane's work counters inside d_ctrs
     kb_pending *lane_pending[KB_MAX_LANES] = {nullptr, nullptr, nullptr, nullptr};  // submitted, rows not yet read back, per lane
-    int prio_lane = 0;                            // priority of the lane streams
-    int prio_bulk = 0;                            // priority of the bulk kernels (decode, gather): the lowest
-    bool prio_split = false;                      // the lane streams run above prio_bulk
+    int prio_lane = 0;                            // priority of the lane streams (above the copy stream's when the device has levels)
     cudaStream_t stream_h = nullptr;              // device -> host copies of KB_OUT_HOST answers (behind the gather's event)
     // per-request results (ReqOut) published by the device into mapped pinned memory: [flag u64 | pad to 64 | rows]
     uint8_t *h_rout = nullptr;
@@ -214,14 +251,13 @@ struct kb_ctx {
     // store
     bool loaded = false;
     StoreDev st{};
-    DBuf d_kslab, d_koff16, d_klen, d_vslab, d_voff16, d_vlen, d_dir;
+    DBuf d_kslab, d_koff16, d_klen, d_vslab, d_voff16, d_vlen, d_dir, d_crev, d_cword;
     uint64_t key_bytes = 0, val_bytes = 0;
     uint32_t max_kv_chunks = 0;  // largest padded [key][value] pair, in 16-byte chunks: sizes the gather's ring buffers
-    uint32_t max_key_chunks = 0; // longest key, in 16-byte chunks: sizes the decode pass's key ring
     // heap + sorted directory (kb_apply_batch): chunks in use at the slab tails, chunks no live record points at, records
     // appended out of key order since the last layout compaction; s_* = the spare directory set the next merge writes
     uint64_t kused16 = 0, vused16 = 0, garbage_k16 = 0, garbage_v16 = 0, displaced = 0, layout_compactions = 0;
-    DBuf s_koff16, s_klen, s_voff16, s_vlen, s_dir;
+    DBuf s_koff16, s_klen, s_voff16, s_vlen, s_dir, s_crev, s_cword;
     bool compact_present = false;
     uint64_t compact_rev = 0;
     // TTL puts: (expire_unix, internal key), ordered by time; ttl_of[key] = the expiry the key currently has (a later put
@@ -230,9 +266,9 @@ struct kb_ctx {
     std::unordered_map<std::string, uint64_t> ttl_of;
 
     // scratch (grow only)
-    DBuf d_bounds, d_bres, d_reqs, d_tiles /* alias into d_reqs */, d_meta, d_tgt, d_agg, d_tcnt /* look-back states */, d_tscan, d_reqout,
+    DBuf d_bounds, d_bres, d_reqs, d_tiles /* alias into d_reqs */, d_tgt, d_agg, d_tcnt /* look-back states */, d_tscan, d_reqout,
         d_sel, d_slot, d_jobs, d_gjobs, d_jobs2, d_gjobs2 /* second job-buffer set */, d_flags,
-        d_ctrs /* work-queue counters, kept at zero between kernels */;
+        d_ctrs /* search counters and the copy kernels' error flag, kept at zero between kernels */;
     HBuf h_stage, h_stage2;
 
     // kb_range_prefetch: bound searches started ahead of the kb_range_batch that will use them (two in flight at most)
@@ -275,12 +311,12 @@ struct kb_ctx {
     uint64_t *h_p2p_out = nullptr;            // pinned: [nranks] gathered cursors, [nranks] min, [nranks+1] status
 
     // profiling
-    int prof_on = 0;  // 0 off, 1 every kernel, 2 only the two HBM-bound kernels (k_decode_lcp, k_gather)
+    int prof_on = 0;  // 0 off, 1 every kernel, 2 only the HBM-bound copy (k_gather)
     std::vector<ProfEntry> prof;
     std::vector<ProfPending> prof_pending;
     std::vector<cudaEvent_t> ev_pool;
     uint64_t launches = 0;
-    bool decode_attr_set = false, gather_attr_set = false, wire_attr_set = false;  // per-context (per-device) kernel attributes
+    bool gather_attr_set = false, wire_attr_set = false;  // per-context (per-device) kernel attributes
 };
 
 struct kb_result {
@@ -344,7 +380,7 @@ void pool_put_host(kb_ctx *ctx, HBuf b);
 
 // profiling: bracket a kernel launch with events when enabled
 int prof_index(kb_ctx *ctx, const char *name);
-static inline bool prof_major(const char *n) { return n[0] == 'k' && n[1] == '_' && ((n[2] == 'd' && n[3] == 'e') || (n[2] == 'g' && n[3] == 'a' && n[8] == 0)); }
+static inline bool prof_major(const char *n) { return strcmp(n, "k_gather") == 0; }
 void prof_begin(kb_ctx *ctx, int idx, uint64_t alg_bytes, cudaStream_t strm);
 void prof_end(kb_ctx *ctx, cudaStream_t strm);
 

@@ -2,26 +2,24 @@
 //
 // Replaces (reference file:line):
 //   storage.Iter over badger            pkg/storage/badger/iter.go:27-98        -> HBM slab + k_search
-//   coder.Decode                        pkg/backend/coder/normal.go:58-70       -> k_decode_lcp
-//   worker.run (range + compact)        pkg/backend/scanner/scanner.go:389-516  -> k_decode_lcp, k_emit, k_place
+//   coder.Decode                        pkg/backend/coder/normal.go:58-70       -> decoded columns (kb_decode.cuh)
+//   worker.run (range + compact)        pkg/backend/scanner/scanner.go:389-516  -> col_meta, k_emit, k_place
 //   commonResultReceiver (limit)        pkg/backend/scanner/receiver.go:62-103  -> k_tile_scan, k_place, k_gather
 //
 // Kernel pipeline for one batch of requests (streams: S2 = bound search, S = main, SG = copy stream):
 //   k_search      [S2] lower_bound of every [start,end) bound in the sorted slab (warp per bound, 32-ary); the only
 //                 step the host waits for before it lays the requests out as tiles
-//   k_decode_lcp  [S] HBM-bound pass: stream the raw internal keys (one bulk-TMA copy per 32-record sub-tile into a
-//                 per-warp shared-memory ring), decode magic/split/revision, visibility, tombstone probe, and the
-//                 common-prefix length with the preceding key -> one 32-bit meta word per record + sub-tile aggregates
-//   k_emit        [S] per tile: segmented "last visible version" scan over the meta words (prev pointer + running
-//                 min-LCP; the cross-tile carry by decoupled look-back) decides which record every key change emits /
-//                 supersedes
+//   k_emit        [S] per tile: every record's meta word from its decoded columns (crev / cword, written with the
+//                 directory: kb_decode.cuh) and the request's read revision, then a segmented "last visible version"
+//                 scan over the meta words (prev pointer + running min-LCP; the cross-tile carry by decoupled look-back)
+//                 decides which record every key change emits / supersedes
 //   k_tile_scan   [S] prefix sums of the per-tile counts / bytes (one CTA per 1024 tiles); k_req_totals: per-request rows
 //   k_place       [S] ordered placement of the selection (limit applied) / ordered victim list
 //   k_req_finalize [S] per-request prefix sums; publishes the per-request rows to mapped pinned memory (the host
 //                 returns device-resident answers on that flag)
 //   k_gather_jobs / k_wire_jobs [S] one copy job per emitted kv + the per-kv view arrays
 //   k_gather / k_wire_copy [SG] bulk-TMA copy of the winners' key+value into the response arena (padded pairs, or
-//                 etcd protobuf elements); overlaps the next batch's k_decode_lcp .. k_place
+//                 etcd protobuf elements); overlaps the next batch's k_emit .. k_place
 #include <algorithm>
 #include <memory>
 
@@ -286,18 +284,23 @@ __device__ __forceinline__ LM lookback_lm(TileState *ts, uint32_t t, uint32_t t0
     return acc;
 }
 
+// meta word of record `rec` for request `req` (col_meta over the record's decoded columns)
+__device__ __forceinline__ uint32_t rec_meta(const StoreDev &st, const ScanMode &mode, const ReqDev &req, uint32_t rec)
+{
+    return col_meta(st.crev[rec], st.cword[rec], mode, req.read_rev, rec == req.lo);
+}
+
 template <bool COMPACT>
-__global__ void __launch_bounds__(256, 8)  // <= 32 registers: must fit beside the persistent CTAs of other batches
-k_emit(StoreDev st, const ReqDev *__restrict__ reqs, const TileDev *__restrict__ tiles, const uint32_t *__restrict__ meta,
+__global__ void __launch_bounds__(256, 8)  // <= 32 registers: must fit beside the gather CTAs and other batches' kernels
+k_emit(StoreDev st, ScanMode mode, const ReqDev *__restrict__ reqs, const TileDev *__restrict__ tiles,
        TileState *__restrict__ ts, unsigned int *__restrict__ ticket, uint32_t *__restrict__ tgt,
-       uint32_t *__restrict__ tail_tgt, uint64_t *__restrict__ tcnt, int wire, unsigned int *__restrict__ decode_ctr)
+       uint32_t *__restrict__ tail_tgt, uint64_t *__restrict__ tcnt)
 {
     __shared__ LM warp_tot[8];
     __shared__ LM carry_s, agg_s;
     __shared__ uint64_t ws2[18];
     __shared__ uint32_t tile_s;
     if (threadIdx.x == 0) tile_s = atomicAdd(ticket, 1u);  // ticket order: every preceding tile has started
-    if (blockIdx.x == 0 && threadIdx.x == 0) *decode_ctr = 0;  // leave k_decode_lcp's work counter at zero
     __syncthreads();
     const uint32_t tix = tile_s;
     const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -308,14 +311,8 @@ k_emit(StoreDev st, const ReqDev *__restrict__ reqs, const TileDev *__restrict__
     const uint32_t base = threadIdx.x * 4;
     const uint32_t flat = tile.flat0 + base;
     uint32_t w[4];
-    {
-        uint4 mw = make_uint4(KB_LCP_INF, KB_LCP_INF, KB_LCP_INF, KB_LCP_INF);
-        if (base < tile.n) mw = *(const uint4 *)(meta + flat);
-        w[0] = base + 0 < tile.n ? mw.x : KB_LCP_INF;
-        w[1] = base + 1 < tile.n ? mw.y : KB_LCP_INF;
-        w[2] = base + 2 < tile.n ? mw.z : KB_LCP_INF;
-        w[3] = base + 3 < tile.n ? mw.w : KB_LCP_INF;
-    }
+#pragma unroll
+    for (int k = 0; k < 4; k++) w[k] = base + k < tile.n ? rec_meta(st, mode, req, tile.rec0 + base + k) : KB_LCP_INF;
     LM mine;
     mine.L = KB_NONE;
     mine.m = KB_LCP_INF;
@@ -338,11 +335,11 @@ k_emit(StoreDev st, const ReqDev *__restrict__ reqs, const TileDev *__restrict__
         carry.m = KB_LCP_INF;
         bool resolved = first_tile;
         if (!first_tile) {
-            // Fast path: the meta words in front of this tile are complete (the decode pass has finished), so the last
-            // PREVOK record is looked for directly in the 256 records before the tile -- 32 per step, nearest first.
-            // Almost every tile ends here without waiting for anybody.
+            // Fast path: the meta word of any record can be computed from its columns, so the last PREVOK record is
+            // looked for directly in the 256 records before the tile -- 32 per step, nearest first.  Almost every tile
+            // ends here without waiting for anybody.
             for (uint32_t back = 0; back < 256 && !resolved; back += 32) {
-                const uint32_t wd = meta[tile.flat0 - 1 - back - lane];  // lane 0 = the record right in front
+                const uint32_t wd = rec_meta(st, mode, req, tile.rec0 - 1 - back - lane);  // lane 0 = the record right in front
                 const unsigned pm = __ballot_sync(FULL, wd & KB_M_PREVOK);
                 const uint32_t k = pm ? (uint32_t)(__ffs(pm) - 1) : 32u;  // nearest PREVOK lane; records nearer than it count
                 const uint32_t mm = __reduce_min_sync(FULL, lane < k ? (wd & KB_M_LCP_MASK) : KB_LCP_INF);
@@ -386,7 +383,7 @@ k_emit(StoreDev st, const ReqDev *__restrict__ reqs, const TileDev *__restrict__
             if (x.L != KB_NONE) {
                 const uint32_t mm = min(x.m, word & KB_M_LCP_MASK);
                 const uint32_t irec = req.lo + (i - req.flat0), prec = req.lo + (x.L - req.flat0);
-                const uint32_t pw = meta[x.L];
+                const uint32_t pw = rec_meta(st, mode, req, prec);
                 const uint32_t kl = st.klen[irec], pkl = st.klen[prec];
                 const bool same = (kl == pkl) && (mm >= kl - 9);
                 if (!same) {
@@ -396,7 +393,7 @@ k_emit(StoreDev st, const ReqDev *__restrict__ reqs, const TileDev *__restrict__
                         } else {
                             t = x.L;
                             cnt++;
-                            aux += kv_resp_bytes(st, prec, wire);
+                            aux += kv_resp_bytes(st, prec, mode.wire);
                         }
                     }
                 } else if (COMPACT && !(pw & KB_M_REV0)) {
@@ -421,15 +418,15 @@ k_emit(StoreDev st, const ReqDev *__restrict__ reqs, const TileDev *__restrict__
             // end of the request's iterator: the trailing prev (scanner.go:503-507)
             uint32_t tt = KB_NONE;
             if (x.L != KB_NONE) {
-                const uint32_t pw = meta[x.L];
+                const uint32_t prec = req.lo + (x.L - req.flat0);
+                const uint32_t pw = rec_meta(st, mode, req, prec);
                 if (!(pw & KB_M_REV0) && !(pw & KB_M_TOMB)) {
                     if (COMPACT) {
                         aux++;
                     } else {
-                        const uint32_t prec = req.lo + (x.L - req.flat0);
                         tt = x.L;
                         cnt++;
-                        aux += kv_resp_bytes(st, prec, wire);
+                        aux += kv_resp_bytes(st, prec, mode.wire);
                     }
                 }
             }
@@ -630,9 +627,9 @@ k_place(StoreDev st, const ReqDev *__restrict__ reqs, const TileDev *__restrict_
 
 // ordered delete calls (compact): per record [superseded prev] [tombstone] [revision record] | [ttl]
 __global__ void __launch_bounds__(256, 8)  // <= 32 registers: must fit beside the persistent CTAs of other batches
-k_place_victims(const ReqDev *__restrict__ reqs, const TileDev *__restrict__ tiles,
-                const uint32_t *__restrict__ meta, const uint32_t *__restrict__ tgt,
-                const uint64_t *__restrict__ tscan, uint32_t *__restrict__ vidx, uint8_t *__restrict__ vcls)
+k_place_victims(StoreDev st, ScanMode mode, const ReqDev *__restrict__ reqs, const TileDev *__restrict__ tiles,
+                const uint32_t *__restrict__ tgt, const uint64_t *__restrict__ tscan, uint32_t *__restrict__ vidx,
+                uint8_t *__restrict__ vcls)
 {
     __shared__ uint64_t ws2[18];
     const TileDev tile = tiles[blockIdx.x];
@@ -647,12 +644,15 @@ k_place_victims(const ReqDev *__restrict__ reqs, const TileDev *__restrict__ til
         w[k] = 0;
     }
     if (base < tile.n) {
-        const uint4 tw = *(const uint4 *)(tgt + flat), mw = *(const uint4 *)(meta + flat);
-        t[0] = tw.x, w[0] = mw.x;
-        if (base + 1 < tile.n) t[1] = tw.y, w[1] = mw.y;
-        if (base + 2 < tile.n) t[2] = tw.z, w[2] = mw.z;
-        if (base + 3 < tile.n) t[3] = tw.w, w[3] = mw.w;
+        const uint4 tw = *(const uint4 *)(tgt + flat);
+        t[0] = tw.x;
+        if (base + 1 < tile.n) t[1] = tw.y;
+        if (base + 2 < tile.n) t[2] = tw.z;
+        if (base + 3 < tile.n) t[3] = tw.w;
     }
+#pragma unroll
+    for (int k = 0; k < 4; k++)
+        if (base + k < tile.n) w[k] = rec_meta(st, mode, req, tile.rec0 + base + k);
 #pragma unroll
     for (int k = 0; k < 4; k++) {
         if (t[k] != KB_NONE) cnt++;
@@ -742,7 +742,7 @@ k_gather_jobs(StoreDev st, const ReqDev *__restrict__ reqs, uint32_t nreq, const
     out.key_len[k] = kl - 13;
     out.val_off[k] = dst_byte + (uint64_t)j.nk * 16;
     out.val_len[k] = vl;
-    out.rev[k] = be64_bytes((const uint8_t *)(st.kslab + j.ksrc16) + kl - 8);
+    out.rev[k] = st.crev[rec];  // an emitted record has a non-zero key revision: the column holds it
     }
 }
 
@@ -758,7 +758,7 @@ constexpr uint32_t GATHER_WARP_CHUNKS = 880;     // shared memory per warp (13.7
 
 __device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
 
-// bounded like dmbar_wait (kb_decode.cuh): a bulk copy that faults never completes its barrier; give up after ~2 s of
+// bounded like dmbar_wait (kb_internal.cuh): a bulk copy that faults never completes its barrier; give up after ~2 s of
 // polling and raise the context's error flag instead of hanging the stream
 __device__ __forceinline__ void mbar_wait_parity(uint64_t *bar, uint32_t parity, unsigned int *err_flag)
 {
@@ -988,13 +988,16 @@ k_key_exists(StoreDev st, const uint4 *__restrict__ bounds, const uint32_t *__re
 // The store is a HEAP of key / value bytes plus a directory sorted by key.  A committed batch appends the bytes of its
 // puts at the slab tails and rebuilds only the directory: every surviving record moves by (#inserts at or before it) -
 // (#deletes before it), every insert lands at (its lower bound) + (#inserts before it) - (#deletes before it).
-// ins_pos / del_pos / rep_pos are ascending; entries are packed like StoreDev::dir.
+// ins_pos / del_pos / rep_pos are ascending; entries are packed like StoreDev::dir.  A surviving record's decoded columns
+// travel with it; k_col_fix then recomputes the entries the batch made stale.
 struct DirArrays {
     uint32_t *koff16;
     uint16_t *klen;
     uint64_t *voff16;
     uint32_t *vlen;
     uint4 *dir;
+    uint64_t *crev;
+    uint32_t *cword;
 };
 
 __device__ __forceinline__ uint32_t lower_bound_u32(const uint32_t *a, uint32_t n, uint32_t v)
@@ -1035,11 +1038,54 @@ k_dir_merge(StoreDev old, const uint32_t *__restrict__ ins_pos, const uint4 *__r
             e.z = r.z;
             e.w = r.w;
         }
-        dir_store(out, i + ib - db, e);
+        const uint32_t at = i + ib - db;
+        dir_store(out, at, e);
+        out.crev[at] = old.crev[i];  // stale for a replaced record or a changed predecessor: k_col_fix rewrites those
+        out.cword[at] = old.cword[i];
     } else if (t < (uint64_t)old.n + n_ins) {
         const uint32_t k = (uint32_t)(t - old.n);
         const uint32_t p = ins_pos[k];
         dir_store(out, p + k - lower_bound_u32(del_pos, n_del, p), ins_ent[k]);
+    }
+}
+
+// The column entries a merge made stale, recomputed from the new directory (`nd`) and the slab bytes.  A surviving
+// record's entry depends on its own key and value and on its predecessor's key, so only these can change:
+//   an inserted record, and the record behind it (its predecessor is new);
+//   the record that takes a deleted record's place (its predecessor was the deleted one's);
+//   a replaced record (its value changed: tombstone flag, revision in the value);
+//   whatever ends up at position 0 (no predecessor).
+// One thread per candidate, O(ops) key reads; a record that is a candidate twice gets the same entry twice.
+__global__ void __launch_bounds__(256)
+k_col_fix(StoreDev nd, const uint32_t *__restrict__ ins_pos, uint32_t n_ins, const uint32_t *__restrict__ del_pos,
+          uint32_t n_del, const uint32_t *__restrict__ rep_pos, uint32_t n_rep, uint64_t *__restrict__ crev,
+          uint32_t *__restrict__ cword)
+{
+    const uint64_t t = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    uint32_t q[2] = {KB_NONE, KB_NONE};
+    if (t < n_ins) {
+        const uint32_t p = ins_pos[t];
+        q[0] = p + (uint32_t)t - lower_bound_u32(del_pos, n_del, p);
+        q[1] = q[0] + 1;
+    } else if (t < (uint64_t)n_ins + n_del) {
+        // the first new record behind the deleted one's place: survivors before it + inserts at or before it
+        const uint32_t k = (uint32_t)(t - n_ins), d = del_pos[k];
+        q[0] = d - k + lower_bound_u32(ins_pos, n_ins, d + 1);
+    } else if (t < (uint64_t)n_ins + n_del + n_rep) {
+        const uint32_t i = rep_pos[t - n_ins - n_del];
+        q[0] = i + lower_bound_u32(ins_pos, n_ins, i + 1) - lower_bound_u32(del_pos, n_del, i);
+    } else if (t == (uint64_t)n_ins + n_del + n_rep) {
+        q[0] = 0;
+    }
+#pragma unroll
+    for (int j = 0; j < 2; j++) {
+        if (q[j] >= nd.n) continue;
+        uint64_t r;
+        uint32_t w;
+        bool less;
+        col_entry(nd, q[j], &r, &w, &less);
+        crev[q[j]] = r;
+        cword[q[j]] = w;
     }
 }
 
@@ -1344,7 +1390,6 @@ int upload_layout(kb_ctx *ctx, const Resolved &R)
     KB_TRY(dbuf_ensure(ctx, ctx->d_reqs, req_bytes + std::max<size_t>(nt, 1) * sizeof(TileDev) + 64));
     ctx->d_tiles.p = (uint8_t *)ctx->d_reqs.p + req_bytes;  // alias into d_reqs (never freed on its own)
     ctx->d_tiles.cap = 0;
-    KB_TRY(dbuf_ensure(ctx, ctx->d_meta, std::max<uint64_t>(R.total_flat, 4) * 4));
     KB_TRY(dbuf_ensure(ctx, ctx->d_tgt, std::max<uint64_t>(R.total_flat, 4) * 4 + nreq * 4 + 16));
     // one zeroed region per batch: [ticket, padded to 64 bytes][one ChunkState per 1024 tiles][one TileState per tile]
     KB_TRY(dbuf_ensure(ctx, ctx->d_tscan, 64 + (std::max<size_t>(nt, 1) / 1024 + 1) * sizeof(ChunkState) +
@@ -1365,69 +1410,6 @@ int upload_layout(kb_ctx *ctx, const Resolved &R)
 }
 
 }  // namespace
-
-// algorithmic key bytes of `n_rec` examined records: the store's average padded key + 10 B of directory fields each
-static inline uint64_t scan_alg_bytes(kb_ctx *ctx, uint64_t n_rec)
-{
-    const uint64_t n = std::max<uint64_t>(ctx->st.n, 1);
-    const uint64_t live16 = ctx->kused16 > ctx->garbage_k16 ? ctx->kused16 - ctx->garbage_k16 : 0;
-    return n_rec * 10 + (uint64_t)((double)live16 * 16.0 / (double)n * (double)n_rec);
-}
-
-// persistent decode pass: one CTA per SM, independent warps; geometry from the store's longest key (kb_decode.cuh)
-template <int MAXW, int KK>
-static int launch_decode_t(kb_ctx *ctx, const DecGeom &g, size_t smem, uint64_t alg_bytes, const ScanMode &mode,
-                           const TileDev *d_tiles, uint32_t *d_meta)
-{
-    static thread_local int attr_dev = -1;
-    static thread_local size_t attr_smem = 0;
-    if (attr_dev != ctx->device || attr_smem < smem) {
-        KB_CUDA(ctx, cudaFuncSetAttribute(k_decode_lcp<MAXW, KK>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(227 * 1024 - 2048)));
-        attr_dev = ctx->device;
-        attr_smem = 227 * 1024 - 2048;
-    }
-    const uint32_t grid = std::min<uint32_t>((g.n_blocks + g.warps - 1) / g.warps, 148);
-    unsigned int *ctrs = (unsigned int *)ctx->d_ctrs.p;  // work counter of this lane, error flag shared
-    // The decode CTA needs (nearly) all of an SM's shared memory, so its grid cannot be distributed while a gather of another
-    // batch is resident; at the stream's priority it would sit at the head of the block scheduler's queue and hold back
-    // every short kernel of the other lane behind it.  It is launched at the lowest priority instead (the lane streams
-    // run above it), so only the bulk kernels wait for each other.
-    cudaLaunchConfig_t cfg;
-    memset(&cfg, 0, sizeof(cfg));
-    cfg.gridDim = dim3(grid);
-    cfg.blockDim = dim3(g.warps * 32);
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = ctx->stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributePriority;
-    attr[0].val.priority = ctx->prio_bulk;
-    cfg.attrs = attr;
-    cfg.numAttrs = ctx->prio_split ? 1 : 0;
-    KB_LAUNCH(ctx, "k_decode_lcp", alg_bytes,
-              (cudaLaunchKernelEx(&cfg, k_decode_lcp<MAXW, KK>, ctx->st, d_tiles, g, mode, d_meta, ctrs + ctx->ctr_base, ctrs + 8)));
-    return KB_OK;
-}
-
-static int launch_decode(kb_ctx *ctx, uint32_t ntiles, uint64_t alg_bytes, const ScanMode &mode, const TileDev *d_tiles,
-                         uint32_t *d_meta)
-{
-    static const uint32_t force_k = getenv("KB_DECODE_K") ? (uint32_t)atoi(getenv("KB_DECODE_K")) : 0;
-    static const uint32_t force_w = getenv("KB_DECODE_WARPS") ? (uint32_t)atoi(getenv("KB_DECODE_WARPS")) : 0;
-    static const uint32_t force_nks = getenv("KB_DECODE_NKS") ? (uint32_t)atoi(getenv("KB_DECODE_NKS")) : 0;
-    size_t smem = 0;
-    const DecGeom g = decode_geometry(ctx->max_key_chunks, ntiles, force_k, force_nks, force_w, &smem);
-#define KB_DEC_K(W)                                                                                     \
-    switch (g.K) {                                                                                      \
-    case 1: return launch_decode_t<W, 1>(ctx, g, smem, alg_bytes, mode, d_tiles, d_meta);               \
-    case 2: return launch_decode_t<W, 2>(ctx, g, smem, alg_bytes, mode, d_tiles, d_meta);               \
-    case 3: return launch_decode_t<W, 3>(ctx, g, smem, alg_bytes, mode, d_tiles, d_meta);               \
-    default: return launch_decode_t<W, 4>(ctx, g, smem, alg_bytes, mode, d_tiles, d_meta);              \
-    }
-    if (g.warps <= 12) { KB_DEC_K(12) }
-    if (g.warps <= 16) { KB_DEC_K(16) }
-    KB_DEC_K(24)
-#undef KB_DEC_K
-}
 
 // bulk-TMA gather of `n_jobs` (upper bound) copy jobs into `arena`
 static int launch_gather(kb_ctx *ctx, cudaStream_t strm, const GatherJob *d_jobs, const uint64_t *d_njobs,
@@ -1450,7 +1432,7 @@ static int launch_gather(kb_ctx *ctx, cudaStream_t strm, const GatherJob *d_jobs
     return KB_OK;
 }
 
-// decode -> emit -> tile scan -> request totals -> (place) for an uploaded layout; everything stays enqueued on
+// emit -> tile scan -> request totals -> (place) for an uploaded layout; everything stays enqueued on
 // ctx->stream.  Range: the selection goes to ctx->d_sel / d_slot; compact: the delete calls go to vidx / vcls.
 static int launch_scan_core(kb_ctx *ctx, const Resolved &R, const ScanMode &mode, bool with_place,
                             uint32_t *vidx = nullptr, uint8_t *vcls = nullptr)
@@ -1459,7 +1441,6 @@ static int launch_scan_core(kb_ctx *ctx, const Resolved &R, const ScanMode &mode
     const uint32_t nreq = (uint32_t)R.reqs.size();
     const ReqDev *d_reqs = (const ReqDev *)ctx->d_reqs.p;
     const TileDev *d_tiles = (const TileDev *)ctx->d_tiles.p;
-    uint32_t *d_meta = (uint32_t *)ctx->d_meta.p;
     uint32_t *d_tgt = (uint32_t *)ctx->d_tgt.p;
     uint32_t *d_tail = d_tgt + std::max<uint64_t>(R.total_flat, 4);
     const uint32_t nchunks = nt / 1024 + 1;
@@ -1468,20 +1449,19 @@ static int launch_scan_core(kb_ctx *ctx, const Resolved &R, const ScanMode &mode
     TileState *d_ts = (TileState *)(d_cs + nchunks);
     uint64_t *d_tcnt = (uint64_t *)ctx->d_tcnt.p, *d_tscan = d_tcnt + (size_t)std::max<uint32_t>(nt, 1) * 2;
     ReqOut *d_rout = (ReqOut *)ctx->d_reqout.p;
-    const uint64_t kbytes = scan_alg_bytes(ctx, R.n_records);
     if (nt) {
         // the ticket and the look-back states start empty
         KB_CUDA(ctx, cudaMemsetAsync(ctx->d_tscan.p, 0, 64 + (size_t)nchunks * sizeof(ChunkState) + (size_t)nt * sizeof(TileState),
                                      ctx->stream));
-        KB_TRY(launch_decode(ctx, nt, kbytes, mode, d_tiles, d_meta));
+        // per record: 12 bytes of decoded columns read, the 4-byte target written
         if (mode.compact) {
-            KB_LAUNCH(ctx, "k_emit_compact", R.n_records * 8,
-                      (k_emit<true><<<nt, 256, 0, ctx->stream>>>(ctx->st, d_reqs, d_tiles, d_meta, d_ts, d_ticket, d_tgt, d_tail,
-                                                                d_tcnt, 0, (unsigned int *)ctx->d_ctrs.p + ctx->ctr_base)));
+            KB_LAUNCH(ctx, "k_emit_compact", R.n_records * 16,
+                      (k_emit<true><<<nt, 256, 0, ctx->stream>>>(ctx->st, mode, d_reqs, d_tiles, d_ts, d_ticket, d_tgt, d_tail,
+                                                                d_tcnt)));
         } else {
-            KB_LAUNCH(ctx, "k_emit", R.n_records * 8,
-                      (k_emit<false><<<nt, 256, 0, ctx->stream>>>(ctx->st, d_reqs, d_tiles, d_meta, d_ts, d_ticket, d_tgt, d_tail,
-                                                                 d_tcnt, mode.wire, (unsigned int *)ctx->d_ctrs.p + ctx->ctr_base)));
+            KB_LAUNCH(ctx, "k_emit", R.n_records * 16,
+                      (k_emit<false><<<nt, 256, 0, ctx->stream>>>(ctx->st, mode, d_reqs, d_tiles, d_ts, d_ticket, d_tgt, d_tail,
+                                                                 d_tcnt)));
         }
         KB_LAUNCH(ctx, "k_tile_scan", (uint64_t)nt * 32,
                   (k_tile_scan<<<nchunks, 256, 0, ctx->stream>>>(d_tcnt, d_tscan, nt, d_cs)));
@@ -1491,8 +1471,8 @@ static int launch_scan_core(kb_ctx *ctx, const Resolved &R, const ScanMode &mode
                   (k_req_totals<<<(nreq + 255) / 256, 256, 0, ctx->stream>>>(d_reqs, nreq, d_tscan, d_rout)));
     if (nt && with_place) {
         if (mode.compact) {
-            KB_LAUNCH(ctx, "k_place_victims", R.n_records * 8,
-                      (k_place_victims<<<nt, 256, 0, ctx->stream>>>(d_reqs, d_tiles, d_meta, d_tgt, d_tscan, vidx, vcls)));
+            KB_LAUNCH(ctx, "k_place_victims", R.n_records * 16,  // columns + targets (the victims are written on top)
+                      (k_place_victims<<<nt, 256, 0, ctx->stream>>>(ctx->st, mode, d_reqs, d_tiles, d_tgt, d_tscan, vidx, vcls)));
         } else {
             KB_LAUNCH(ctx, "k_place", R.n_records * 4,
                       (k_place<<<nt, 256, 0, ctx->stream>>>(ctx->st, d_reqs, d_tiles, d_tgt, d_tail, d_tscan,
@@ -1828,7 +1808,7 @@ static int pending_harvest(kb_ctx *ctx, kb_pending *P)
         if (P->harvest_rc != KB_OK) return P->harvest_rc;
         memcpy(P->rout.data(), P->h_rout + 64, P->nreq * sizeof(ReqOut));
         if (*(volatile uint64_t *)(P->h_rout + 8) != 0)
-            return P->harvest_rc = kb_fail(ctx, KB_ECUDA, "range scan: a bulk copy of the decode pass never completed");
+            return P->harvest_rc = kb_fail(ctx, KB_ECUDA, "range scan: a bulk copy of the answer never completed");
     }
     return KB_OK;
 }
@@ -2432,10 +2412,10 @@ extern "C" int kb_compact_view_get(const kb_result *res, kb_compact_view *v)
 // Round 1 rebuilt both slabs and merged the whole directory on the host for every batch (O(store bytes)).  Now the
 // store is a heap + a sorted directory: the bytes of the batch's puts are appended at the slab tails (a value that
 // replaces an existing key leaves the old bytes behind as garbage; the key bytes are reused), and only the directory
-// (34 bytes per record) is rebuilt, on the device, by k_dir_merge.  The decode pass stages a step's keys with one bulk
-// copy when they lie within one ring slot of each other and reads them in place otherwise, so records appended out of
-// key order cost a slower step, not a wrong one.  When more than 1/32 of the records are out of place, or a quarter of a
-// slab is garbage, store_compact_layout rewrites the slabs contiguously in key order (O(store), amortised O(1) per op).
+// (46 bytes per record with the decoded columns) is rebuilt, on the device, by k_dir_merge + k_col_fix.  Records
+// appended out of key order cost the copy kernels scattered reads, not wrong answers.  When more than 1/32 of the
+// records are out of place, or a quarter of a slab is garbage, store_compact_layout rewrites the slabs contiguously in
+// key order (O(store), amortised O(1) per op).
 // ------------------------------------------------------------------------------------------------
 namespace {
 struct ApplyOp {
@@ -2468,6 +2448,8 @@ static int dir_spare_ensure(kb_ctx *ctx, uint64_t n)
     KB_TRY(dbuf_ensure(ctx, ctx->s_voff16, (n + 1) * 8));
     KB_TRY(dbuf_ensure(ctx, ctx->s_vlen, (n + 1) * 4));
     KB_TRY(dbuf_ensure(ctx, ctx->s_dir, (n + 1) * 16));
+    KB_TRY(dbuf_ensure(ctx, ctx->s_crev, (n + 1) * 8));
+    KB_TRY(dbuf_ensure(ctx, ctx->s_cword, (n + 1) * 4));
     return KB_OK;
 }
 
@@ -2478,11 +2460,15 @@ static void dir_swap(kb_ctx *ctx, uint64_t n)
     std::swap(ctx->d_voff16, ctx->s_voff16);
     std::swap(ctx->d_vlen, ctx->s_vlen);
     std::swap(ctx->d_dir, ctx->s_dir);
+    std::swap(ctx->d_crev, ctx->s_crev);
+    std::swap(ctx->d_cword, ctx->s_cword);
     ctx->st.koff16 = (const uint32_t *)ctx->d_koff16.p;
     ctx->st.klen = (const uint16_t *)ctx->d_klen.p;
     ctx->st.voff16 = (const uint64_t *)ctx->d_voff16.p;
     ctx->st.vlen = (const uint32_t *)ctx->d_vlen.p;
     ctx->st.dir = (const uint4 *)ctx->d_dir.p;
+    ctx->st.crev = (const uint64_t *)ctx->d_crev.p;
+    ctx->st.cword = (const uint32_t *)ctx->d_cword.p;
     ctx->st.kslab = (const uint4 *)ctx->d_kslab.p;
     ctx->st.vslab = (const uint4 *)ctx->d_vslab.p;
     ctx->st.n = (uint32_t)n;
@@ -2530,6 +2516,9 @@ int store_compact_layout(kb_ctx *ctx)
                                                                (const uint64_t *)ctx->s_voff16.p, (uint4 *)nk.p, (uint4 *)nv.p)));
         cudaMemcpyAsync(ctx->s_klen.p, ctx->st.klen, n * 2, cudaMemcpyDeviceToDevice, ctx->stream);
         cudaMemcpyAsync(ctx->s_vlen.p, ctx->st.vlen, n * 4, cudaMemcpyDeviceToDevice, ctx->stream);
+        // directory order does not change: the decoded columns stay valid
+        cudaMemcpyAsync(ctx->s_crev.p, ctx->st.crev, n * 8, cudaMemcpyDeviceToDevice, ctx->stream);
+        cudaMemcpyAsync(ctx->s_cword.p, ctx->st.cword, n * 4, cudaMemcpyDeviceToDevice, ctx->stream);
     }
     cudaError_t e = cudaStreamSynchronize(ctx->stream);  // the host vectors die here; the old slabs are released below
     if (e != cudaSuccess) {
@@ -2676,7 +2665,7 @@ static int apply_batch_locked(kb_ctx *ctx, const kb_write_op *ops, uint64_t n_op
     std::vector<uint4> ins_ent, rep_ent;
     std::vector<uint8_t> kimg, vimg;  // images of the appended key / value chunks
     uint64_t ktail = ctx->kused16, vtail = ctx->vused16, garbage_k = 0, garbage_v = 0;
-    uint32_t max_k = ctx->max_key_chunks, max_kv = ctx->max_kv_chunks;
+    uint32_t max_kv = ctx->max_kv_chunks;
     auto append = [](std::vector<uint8_t> &img, const std::string &b) {
         const size_t at = img.size(), n16 = (b.size() + 15) / 16;
         img.resize(at + n16 * 16, 0);
@@ -2701,7 +2690,6 @@ static int apply_batch_locked(kb_ctx *ctx, const kb_write_op *ops, uint64_t n_op
                 ins_ent.push_back(entry(ktail, m[i].key.size(), vo, m[i].val.size()));
                 ktail += append(kimg, m[i].key);
             }
-            max_k = std::max<uint32_t>(max_k, (uint32_t)nk);
             max_kv = std::max<uint32_t>(max_kv, (uint32_t)std::min<uint64_t>(nk + nv, 0xFFFFFFFFu));
         } else if (exists[i]) {
             del_pos.push_back(pos[i]);
@@ -2738,7 +2726,7 @@ static int apply_batch_locked(kb_ctx *ctx, const kb_write_op *ops, uint64_t n_op
     if (!vimg.empty())
         KB_CUDA(ctx, cudaMemcpyAsync((uint8_t *)ctx->d_vslab.p + ctx->vused16 * 16, h2 + kimg.size(), vimg.size(),
                                      cudaMemcpyHostToDevice, ctx->stream));
-    // key_less / decode read up to three chunks past a key: keep the slack behind the tails zero
+    // key_less reads up to three chunks past a key: keep the slack behind the tails zero
     KB_CUDA(ctx, cudaMemsetAsync((uint8_t *)ctx->d_kslab.p + ktail * 16, 0, 64, ctx->stream));
     KB_CUDA(ctx, cudaMemsetAsync((uint8_t *)ctx->d_vslab.p + vtail * 16, 0, 64, ctx->stream));
     KB_CUDA(ctx, cudaMemcpyAsync(ctx->d_bounds.p, ht, tab_bytes - 64, cudaMemcpyHostToDevice, ctx->stream));
@@ -2751,11 +2739,28 @@ static int apply_batch_locked(kb_ctx *ctx, const kb_write_op *ops, uint64_t n_op
     out.voff16 = (uint64_t *)ctx->s_voff16.p;
     out.vlen = (uint32_t *)ctx->s_vlen.p;
     out.dir = (uint4 *)ctx->s_dir.p;
+    out.crev = (uint64_t *)ctx->s_crev.p;
+    out.cword = (uint32_t *)ctx->s_cword.p;
     const uint64_t threads = N + n_ins;
-    KB_LAUNCH(ctx, "k_dir_merge", (N + N2) * 34,
+    KB_LAUNCH(ctx, "k_dir_merge", (N + N2) * 46,
               (k_dir_merge<<<(unsigned)((threads + 255) / 256), 256, 0, ctx->stream>>>(ctx->st, d_ins_pos, d_ins_ent, (uint32_t)n_ins,
                                                                                        d_del_pos, (uint32_t)n_del, d_rep_pos,
                                                                                        d_rep_ent, (uint32_t)n_rep, out)));
+    // the stale column entries, from the new directory: per candidate two keys, two directory entries, one value probe
+    StoreDev nd = ctx->st;
+    nd.koff16 = out.koff16;
+    nd.klen = out.klen;
+    nd.voff16 = out.voff16;
+    nd.vlen = out.vlen;
+    nd.dir = out.dir;
+    nd.crev = out.crev;
+    nd.cword = out.cword;
+    nd.n = (uint32_t)N2;
+    const uint64_t n_fix = 2 * n_ins + n_del + n_rep + 1;
+    const uint64_t mean_key = ktail * 16 / std::max<uint64_t>(N2, 1);
+    KB_LAUNCH(ctx, "k_col_fix", n_fix * (2 * mean_key + 2 * 14 + 16 + 12),
+              (k_col_fix<<<(unsigned)((n_ins + n_del + n_rep + 1 + 255) / 256), 256, 0, ctx->stream>>>(
+                  nd, d_ins_pos, (uint32_t)n_ins, d_del_pos, (uint32_t)n_del, d_rep_pos, (uint32_t)n_rep, out.crev, out.cword)));
     e = cudaStreamSynchronize(ctx->stream);  // the staging buffers are reused by the next call
     if (e != cudaSuccess) {
         ctx->loaded = false;
@@ -2770,7 +2775,6 @@ static int apply_batch_locked(kb_ctx *ctx, const kb_write_op *ops, uint64_t n_op
     ctx->garbage_k16 += garbage_k;
     ctx->garbage_v16 += garbage_v;
     ctx->displaced += n_ins;
-    ctx->max_key_chunks = max_k;
     ctx->max_kv_chunks = max_kv;
     if (ctx->displaced > std::max<uint64_t>(4096, N2 / 32) || ctx->garbage_k16 * 4 > ktail || ctx->garbage_v16 * 4 > vtail)
         KB_TRY(store_compact_layout(ctx));

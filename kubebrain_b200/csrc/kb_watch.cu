@@ -95,7 +95,12 @@ struct TabDev {
 // control words of one match (gstate: [gcnt G+1][gfill G+1][ctl 16])
 enum { FC_NONMONO = 0, FC_CURSOR = 1, FC_NLARGE = 2, FC_NMED = 3, FC_ARRIVE = 4, FC_GEN = 5, FC_DONE = 6, FC_ABORT = 7, FC_WORDS = 16 };
 constexpr unsigned long long FAN_UNSET = ~0ull, FAN_BUSY = ~0ull - 1;
-constexpr uint32_t FAN_THREADS = 384;  // one CTA per SM, < 28 k registers (fits beside the decode CTA or the two gather CTAs), < 2 KiB of shared memory (see fan_grid_sync)
+// One CTA per SM, < 2 KiB of shared memory (see fan_grid_sync).  Registers: 384 threads x 80 (k_fanout's cap, no spill)
+// = 30 720; its neighbours on an SM are the scan context's two gather CTAs (2 x 256 x 32 = 16 384) and the short scan
+// kernels (256 x 32 = 8 192 per CTA): 30 720 + 16 384 + 2 x 8 192 = 63 488 of 65 536.  Measured on a B200 (1 000 W,
+// 1 965 MHz max SM clock, bench step, 3 runs each): cap 64 (28 B spilled) 4.26-4.52 G events/s, 72 (20 B) 4.55-4.59,
+// 80 4.62-4.66 (profiles/r03_fanout_cap_ab.txt).
+constexpr uint32_t FAN_THREADS = 384;
 constexpr uint32_t BM_WORDS = 256;   // 8192 event indices per shared-memory window (1 KiB).  The scan context's two gather
                                      // CTAs leave ~6 KiB of an SM's shared memory (every resident CTA also costs 1 KiB of
                                      // reserve): with a 4 KiB window here NOTHING else of the scan context -- not even the
@@ -618,7 +623,7 @@ __device__ __forceinline__ uint64_t fan_now_ns()
     return t;
 }
 
-__global__ void __maxnreg__(64)  // 384 threads x 64 registers: leaves the scan context's decode CTA its 12 warps x 80 on the same SM
+__global__ void __maxnreg__(80)  // 384 threads x 80 registers, see FAN_THREADS
 k_fanout(EvDev ev, TabDev tb, FanScratch sc)
 {
     // phase timestamps of CTA 0 (profiling: kb_prof_read reports them as fan:P1 .. fan:finish when profiling is on)

@@ -122,7 +122,7 @@ k_wire_jobs(StoreDev st, const ReqDev *__restrict__ reqs, uint32_t nreq, const u
         const uint64_t E = arena_base[q] + slot[s];
         const uint32_t kl = st.klen[rec], vl = st.vlen[rec];
         const uint32_t ksrc16 = st.koff16[rec];
-        const uint64_t rev = be64_bytes((const uint8_t *)(st.kslab + ksrc16) + kl - 8);
+        const uint64_t rev = st.crev[rec];  // an emitted record has a non-zero key revision: the column holds it
         const WireSizes ws = wire_sizes(kl - 13, vl, rev, wire);
         __align__(16) uint8_t h1[32], h2[32];
         uint32_t n1, n2;
@@ -337,7 +337,7 @@ __device__ __forceinline__ uint32_t wsmem_u32(const void *p) { return (uint32_t)
 
 __device__ __forceinline__ void wmbar_wait(uint64_t *bar, uint32_t parity, unsigned int *err_flag)
 {
-    dmbar_wait(bar, parity, err_flag);  // bounded: see kb_decode.cuh
+    dmbar_wait(bar, parity, err_flag);  // bounded: see kb_internal.cuh
 }
 
 constexpr int WIRE_MAX_STAGES = 8;

@@ -1,5 +1,5 @@
 #!/bin/bash
-# the two bench lines of the committed state on one box (tools/final_measure.sh has the tests and the ncu passes)
+# the bench lines of the committed state on one box: the reference arm, the default line and the --in-flight 1 line
 mkdir -p gpurun_out
 timeout -s KILL 900 python bench.py --impl reference --steps 3 --warmup 1 > gpurun_out/final_bench_reference.json 2> gpurun_out/final_bench_reference.err
 timeout -s KILL 1200 python bench.py > gpurun_out/final_bench.json 2> gpurun_out/final_bench.err

@@ -4,7 +4,6 @@ mkdir -p gpurun_out
 make -C kubebrain_b200/csrc 2>&1 | tail -2
 echo "== quick tests"; timeout -s KILL 900 python -m pytest tests/test_gpu_round2.py tests/test_cpp_host.py -x -q -m gpu -k "not geometries" 2>&1 | tail -6 | tee gpurun_out/t_r2.log
 timeout -s KILL 600 python -m pytest tests/test_gpu_parity.py -x -q -k "fanout or config3 or watch or compact or config4_shape or fuzz_range or config2_shape or range_table" 2>&1 | tail -8 | tee gpurun_out/t_fanout.log
-echo "== decode sweep"; timeout -s KILL 1200 python tools/decode_sweep.py 2>&1 | tee gpurun_out/decode_sweep.txt
 echo "== bench"; timeout -s KILL 1200 python bench.py --steps 20 --warmup 5 > gpurun_out/bench.json 2> gpurun_out/bench.err; echo "rc=$?"; tail -c 1500 gpurun_out/bench.err
 python - <<'PY'
 import json

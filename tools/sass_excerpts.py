@@ -9,7 +9,7 @@ import sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 SO = os.path.join(ROOT, "kubebrain_b200", "libkbb200.so")
 OUT = os.path.join(ROOT, "profiles", "r02_sass_excerpts.txt")
-WANT = ["k_gather", "k_decode_lcpILi12ELi1E", "k_decode_lcpILi16ELi2E", "k_wire_copy", "k_fanout", "k_emitILb0", "k_dir_merge",
+WANT = ["k_gather", "k_wire_copy", "k_fanout", "k_emitILb0", "k_dir_merge",
         "k_cursor_p2p"]
 PATS = ["UBLKCP", "SYNCS", "FENCE", "LDG.E.128", "STG.E.128", "LDS.128", "REDUX", "VOTE", "MATCH", "SHFL", "ATOM", "RED.",
         "NANOSLEEP", "MEMBAR", "CCTL"]
